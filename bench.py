@@ -40,6 +40,10 @@ UNIT = "segments/s"
 # neighbour ids + 16 B flux read-modify-write; per flying track 61 B read + 28 B written
 BYTES_PER_SEGMENT = 128
 BYTES_PER_TRACK = 89
+# --dump-outputs writes at most this many flux entries and particles (52 MiB of float64 with their
+# indices); larger meshes and batches are sampled
+DUMP_ELEMENTS = 1 << 21
+DUMP_PARTICLES = 1 << 19
 
 
 def env_int(name, default):
@@ -72,6 +76,25 @@ def recorded_traffic():
                 "source": "profiles/traffic.json (%s)" % t.get("source", "ncu capture")}
     except Exception:
         return None
+
+
+def dump_outputs(out_dir, flux, elem_ids, positions):
+    """What a caller reads after the last timed move -- the flux tally and each particle's parent element
+    and position -- as float64 DIR/<name>.npy, so that two builds can be compared output for output.
+    Arrays longer than DUMP_ELEMENTS / DUMP_PARTICLES are cut to a fixed seeded sample whose indices
+    are written beside them."""
+    import numpy as np
+
+    def sample(n, k, seed):
+        return np.arange(n) if n <= k else np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+
+    e = sample(len(flux), DUMP_ELEMENTS, 1)
+    p = sample(len(elem_ids), DUMP_PARTICLES, 2)
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"flux": flux[e], "flux_element_index": e, "elem_ids": elem_ids[p], "positions": positions[p],
+              "particle_index": p}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def bind_to_gpu_node(torch, index):
@@ -198,6 +221,8 @@ def run_reference(args, rank):
     for o, d, f, w in batches:
         orc.MoveToNextLocation(o.reshape(-1), d.reshape(-1), f, w)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, orc.flux, orc.elem_ids, orc.positions)
     segs = orc.n_segments - s0
     value = segs / dt
     sample = (f"first {n} particles of the {args.config} batch per step ({args.steps} steps, "
@@ -261,8 +286,10 @@ class GpuArm:
             self.dist.all_reduce(t, op=getattr(self.dist.ReduceOp, op))
         return [float(x) for x in t]
 
-    def measure(self, cfg_name, n, steps, warmup, e2e=True, e2e_modes=False, clocks=False, scaling="weak"):
-        """Device-resident and end-to-end throughput of `cfg_name` with n particles on this rank."""
+    def measure(self, cfg_name, n, steps, warmup, e2e=True, e2e_modes=False, clocks=False, scaling="weak",
+                dump_dir=None):
+        """Device-resident and end-to-end throughput of `cfg_name` with n particles on this rank; with
+        dump_dir, rank 0 writes the device-resident engine's results there (dump_outputs)."""
         from pumiumtally_b200.tally import PumiTally
         from pumiumtally_b200.workload import CONFIGS, SyntheticWorkload
 
@@ -354,12 +381,15 @@ class GpuArm:
         kernel_ms = st1["kernel_ms"] - st0["kernel_ms"]
         ms_max = self.reduce([ms], "MAX")[0]
         total_segs, total_tracks = self.reduce([float(segs), float(tracks)], "SUM")
+        flux = eng.flux  # collective after a reduce-scatter exchange: every rank reads it
+        if dump_dir and rank == 0:
+            dump_outputs(dump_dir, flux, eng.elem_ids, eng.positions)
         out = {
             "config": cfg_name, "particles_per_gpu": n, "n_gpus": world, "scaling": scaling, "steps": steps,
             "value": total_segs / (ms_max * 1e-3), "ms_per_step": ms_max / steps,
             "segments_per_track": total_segs / max(total_tracks, 1.0), "lost": int(st1["lost"]),
             "relocation_crossings_per_step": (st1["relocations"] - st0["relocations"]) / max(steps, 1),
-            "flux_sum": float(eng.flux.sum()), "variant": eng.get_option("variant"),
+            "flux_sum": float(flux.sum()), "variant": eng.get_option("variant"),
             "gpu_launches": eng.get_option("launches") - launches0,  # kernels the engine launched in the timed region
             "allreduce_ms": (eng.get_option("allreduce_us") / 1e3) if world > 1 else None,  # the batch-end exchange
             "allreduce_bytes": 8 * eng.num_elements if world > 1 else None,
@@ -506,7 +536,7 @@ def run_gpu(args, rank, local_rank, world):
     if world == 1 and cfg.get("gpus", 1) > 1 and not args.particles:
         n = cfg["particles"] // cfg["gpus"] if args.per_gpu_share else cfg["particles"]
     main = arm.measure(args.config, n, args.steps, args.warmup, e2e=not args.no_e2e,
-                       e2e_modes=not args.no_e2e_modes, clocks=True)
+                       e2e_modes=not args.no_e2e_modes, clocks=True, dump_dir=args.dump_outputs)
 
     # ---- the multi-GPU configurations BASELINE.json names, measured beside the headline ----------
     # c4 on 4 GPUs (1 M particles / 4), c5 on 8 GPUs (100 M particles / 8), and c5 strong scaling
@@ -590,7 +620,12 @@ def main():
                     help="skip the extra blocks when the headline measurement has already taken this long")
     ap.add_argument("--no-extra", action="store_true",
                     help="N>1: skip the extra blocks (c4 on 4 GPUs, c5 on 8 GPUs, c5 strong scaling)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the flux and the particles' elements and positions "
+                         "(float64 .npy, seeded samples of large arrays, at most 64 MiB) to DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
     rank, local_rank, world = env_int("RANK", 0), env_int("LOCAL_RANK", 0), env_int("WORLD_SIZE", 1)
     if args.impl == "reference":

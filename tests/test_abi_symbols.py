@@ -3,6 +3,7 @@ symbol include/pumitally_c.h declares, and export the Itanium-mangled members
 of pumitally::PumiTally exactly as the reference header declares them
 (reference: src/pumitally/PumiTally.h:34-107)."""
 import ctypes
+import json
 import os
 import re
 import subprocess
@@ -73,14 +74,9 @@ def test_facade_header_is_layout_compatible(tmp_path, lib_path):
     und = subprocess.check_output(["nm", "-u", str(obj)], text=True)
     needed = {l.split()[-1] for l in und.splitlines() if "pumitally" in l}
     assert needed == {s for s in REF_MANGLED if "C2" not in s and "D2" not in s}, needed
-    ref_hdr = "/root/reference/src/pumitally"
-    if os.path.isdir(ref_hdr):  # only in the build container: same TU against the reference header
-        src2 = tmp_path / "use_ref.cpp"
-        src2.write_text("#include <string>\n" + src.read_text().replace('"pumitally/PumiTally.h"', '"PumiTally.h"'))
-        obj2 = tmp_path / "use_ref.o"
-        subprocess.check_call(["/usr/bin/g++", "-std=c++17", "-c", "-I", ref_hdr, str(src2), "-o", str(obj2)])
-        und2 = subprocess.check_output(["nm", "-u", str(obj2)], text=True)
-        assert needed == {l.split()[-1] for l in und2.splitlines() if "pumitally" in l}
+    # the same TU compiled against the reference header needs exactly these symbols
+    with open(os.path.join(ROOT, "tests", "golden", "reference_facade_symbols.json")) as f:
+        assert needed == set(json.load(f)["undefined"])
 
 
 def test_no_gpu_means_loud_failure(lib_path):
