@@ -22,7 +22,6 @@ LIB_EXP = os.path.join(LIBDIR, "libpumitally_exp.so")  # product + measured alte
 SOURCES = [
     "walk_kernels.cu",
     "bin_kernels.cu",
-    "l2_partitions.cu",
     "engine.cu",
     "host_stage.cpp",
     "tet_mesh.cpp",

@@ -28,14 +28,10 @@ __device__ __forceinline__ int32_t cell_of(const SeedGrid &g, double x, double y
 }
 
 // pass 1: cell of every flying particle of [begin,end) + histogram
-// origin == nullptr: every particle starts this move where it is (the host path that patches
-// re-sourced particles beforehand); the key is then the stored position
-// mid != nullptr: the key is the cell of the track's midpoint (origin + dest) / 2 instead of its start:
-// the tets a track touches then lie within half a track length of the key cell, which shrinks the halo of
-// the in-flight window (the working set that has to stay in L2) -- profiles/r02/README.md, c5.
+// origin == nullptr: every particle starts this move where it is; the key is then the stored position
 __global__ void bin_count_kernel(SeedGrid g, const double *__restrict__ origin, const ParticleState *__restrict__ state,
-                                 const double *__restrict__ mid, const int8_t *__restrict__ flying, int32_t begin,
-                                 int32_t end, int32_t *__restrict__ pcell, unsigned int *__restrict__ count) {
+                                 const int8_t *__restrict__ flying, int32_t begin, int32_t end,
+                                 int32_t *__restrict__ pcell, unsigned int *__restrict__ count) {
   const int i = begin + blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= end) return;
   const bool fly = flying ? (flying[i] == 1) : true;
@@ -47,10 +43,6 @@ __global__ void bin_count_kernel(SeedGrid g, const double *__restrict__ origin, 
     } else {
       const ParticleState s = load_state(state + i);
       x = s.x; y = s.y; z = s.z;
-    }
-    if (mid) {
-      const double mx = mid[3 * (size_t)i], my = mid[3 * (size_t)i + 1], mz = mid[3 * (size_t)i + 2];
-      if (all_finite(mx, my, mz)) { x = 0.5 * (x + mx); y = 0.5 * (y + my); z = 0.5 * (z + mz); }
     }
     c = cell_of(g, x, y, z);
     atomicAdd(count + c, 1u);
@@ -161,13 +153,13 @@ cudaError_t launch_bin_pack_particles(const SeedGrid &g, const double *origin, c
                                       const double *weights, const int8_t *flying, const ParticleState *state,
                                       int32_t begin, int32_t end, int32_t *pcell, unsigned int *count,
                                       unsigned int *sums, PackedRow *rows, unsigned int *work_count,
-                                      bool midpoint_key, cudaStream_t stream) {
+                                      cudaStream_t stream) {
   const int32_t ncell = g.nx * g.ny * g.nz;
   const int n = end - begin;
   if (n <= 0) return cudaMemsetAsync(work_count, 0, sizeof(unsigned int), stream);
   cudaError_t e = cudaMemsetAsync(count, 0, size_t(ncell) * sizeof(unsigned int), stream);
   if (e != cudaSuccess) return e;
-  bin_count_kernel<<<(n + 255) / 256, 256, 0, stream>>>(g, origin, state, midpoint_key ? dest : nullptr, flying, begin, end, pcell, count);
+  bin_count_kernel<<<(n + 255) / 256, 256, 0, stream>>>(g, origin, state, flying, begin, end, pcell, count);
   const int nb = (ncell + kScanBlock - 1) / kScanBlock;
   scan_block_kernel<<<nb, 256, 0, stream>>>(count, sums, ncell);
   scan_sums_kernel<<<1, 1024, 0, stream>>>(sums, nb, work_count);
@@ -179,7 +171,7 @@ cudaError_t launch_bin_pack_particles(const SeedGrid &g, const double *origin, c
 // count: [ncell] scratch (zeroed here), sums: [ceil(ncell/1024)] scratch, order: [end-begin]
 // compact output, work_count: device scalar receiving the number of flying particles.
 cudaError_t launch_bin_particles(const SeedGrid &g, const double *origin, const ParticleState *state,
-                                 const double *mid, const int8_t *flying, int32_t begin, int32_t end, int32_t *pcell, unsigned int *count,
+                                 const int8_t *flying, int32_t begin, int32_t end, int32_t *pcell, unsigned int *count,
                                  unsigned int *sums, int32_t *order, unsigned int *work_count,
                                  cudaStream_t stream) {
   const int32_t ncell = g.nx * g.ny * g.nz;
@@ -187,7 +179,7 @@ cudaError_t launch_bin_particles(const SeedGrid &g, const double *origin, const 
   if (n <= 0) return cudaMemsetAsync(work_count, 0, sizeof(unsigned int), stream);
   cudaError_t e = cudaMemsetAsync(count, 0, size_t(ncell) * sizeof(unsigned int), stream);
   if (e != cudaSuccess) return e;
-  bin_count_kernel<<<(n + 255) / 256, 256, 0, stream>>>(g, origin, state, mid, flying, begin, end, pcell, count);
+  bin_count_kernel<<<(n + 255) / 256, 256, 0, stream>>>(g, origin, state, flying, begin, end, pcell, count);
   const int nb = (ncell + kScanBlock - 1) / kScanBlock;
   scan_block_kernel<<<nb, 256, 0, stream>>>(count, sums, ncell);
   scan_sums_kernel<<<1, 1024, 0, stream>>>(sums, nb, work_count);

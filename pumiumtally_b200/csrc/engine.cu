@@ -2,8 +2,6 @@
 #include "engine.hpp"
 
 #include <sys/mman.h>
-#include <sys/syscall.h>
-#include <unistd.h>
 
 #include <algorithm>
 #include <atomic>
@@ -79,7 +77,7 @@ Engine::Engine(HostMesh &&mesh, int32_t num_particles, int device)
   dev_alloc(&d_stats_, 1, "stats");
   dev_alloc(&d_initial_weight_, 1, "initial weight");
   cuda_or_throw(cudaMemset(d_initial_weight_, 0, sizeof(double)), "memset");
-  dev_alloc(&d_tickets_, 2 * kTicketRing, "tickets");  // second half: the other L2 partition's tickets (die split)
+  dev_alloc(&d_tickets_, kTicketRing, "tickets");
   dev_alloc(&d_pcell_, N, "particle cells");
   dev_alloc(&d_order_, N, "processing order");
   dev_alloc(&d_work_count_, kTicketRing, "work counts");
@@ -99,9 +97,6 @@ Engine::Engine(HostMesh &&mesh, int32_t num_particles, int device)
            "shortcut; option seed_grid=2 forces it)\n");
   variant_ = choose_variant();
   if (const char *env = std::getenv("PUMITALLY_REGISTER_HOST")) register_host_ = std::atoi(env) != 0;
-  if (const char *env = std::getenv("PUMITALLY_DIE_SPLIT")) {
-    if (std::atoi(env) != 0) set_option("die_split", 1);
-  }
   // the packed records are only needed on the device from here on
   std::vector<TetRecord>().swap(mesh_.records);
   printf("[INFO] pumitally-b200: %lld elements, %d particles on CUDA device %d\n",
@@ -156,10 +151,6 @@ Engine::~Engine() {
   for (auto &t : timers_busy_) { cudaEventDestroy(t.a); cudaEventDestroy(t.b); }
   for (auto &e : chunk_events_) cudaEventDestroy(e);
   stager_.reset();
-  if (h_pos_) { cudaHostUnregister(h_pos_); free(h_pos_); }
-  if (d2h_) cudaStreamDestroy(d2h_);
-  for (auto &e : pos_events_) cudaEventDestroy(e);
-  for (auto &e : walk_events_) cudaEventDestroy(e);
   if (stage_base_) {
     if (stage_registered_) { cudaHostUnregister(stage_base_); free(stage_base_); }
     else cudaFreeHost(stage_base_);
@@ -281,25 +272,6 @@ void Engine::begin_move() {
   }
 }
 
-// Re-sourced particles of the pinned-caller host path: phase 1 for the listed particles only.
-int Engine::relocate_patches(const PatchEntry *d_list, int32_t count, cudaStream_t stream) {
-  if (count <= 0) return 0;
-  WalkParams p{};
-  p.tets = d_tets_;
-  p.flux = d_flux_;
-  p.state = d_state_;
-  p.begin = 0;
-  p.end = n_;
-  p.max_iters = max_iters_ > 0 ? max_iters_ : int32_t(std::min<int64_t>(mesh_.ntets + 16, INT_MAX));
-  p.stats = d_stats_;
-  p.grid = grid_;
-  p.cx = mesh_.center[0]; p.cy = mesh_.center[1]; p.cz = mesh_.center[2];
-  if (!use_seed_grid_) p.grid.cell_tet = nullptr;
-  PTB_CUDA_OK(launch_relocate_patches(p, d_list, count, d_flying_, stream));
-  ++launches_;
-  return 0;
-}
-
 int Engine::launch_range(const double *d_origin, const double *d_dest, const int8_t *d_flying,
                          const double *d_weights, int32_t begin, int32_t end, cudaStream_t stream,
                          bool timed) {
@@ -362,12 +334,6 @@ int Engine::launch_range_into(double *d_flux, const double *d_origin, const doub
   p.cx = mesh_.center[0]; p.cy = mesh_.center[1]; p.cz = mesh_.center[2];
   if (!use_seed_grid_) p.grid.cell_tet = nullptr;
   p.work_counter = d_tickets_ + (ticket_next_++ % kTicketRing);
-  if (die_split_ && die0_sms_ > 0) {  // sorted kernels: each L2 partition's SMs on their own end of the sequence
-    for (int i = 0; i < 8; ++i) p.die_mask[i] = die_mask_[i];
-    p.die0_sms = die0_sms_;
-    p.nsms = nsms_;
-    p.work_counter2 = p.work_counter + kTicketRing;
-  }
   auto aligned16 = [](const void *q) { return (reinterpret_cast<uintptr_t>(q) & 15u) == 0; };
   p.bulk_ok = (begin % 16 == 0) && aligned16(d_origin) && aligned16(d_dest) && aligned16(d_flying) &&
               aligned16(d_weights);
@@ -408,7 +374,7 @@ int Engine::launch_range_into(double *d_flux, const double *d_origin, const doub
     SeedGrid bin_grid = grid_;
     if (!morton_) bin_grid.cell_rank = nullptr;
     PTB_CUDA_OK(launch_bin_pack_particles(bin_grid, d_origin, d_dest, d_weights, d_flying, d_state_, begin, end,
-                                          d_pcell_, d_cell_count_, d_cell_sums_, d_rows_ + begin, wc, bin_midpoint_, stream));
+                                          d_pcell_, d_cell_count_, d_cell_sums_, d_rows_ + begin, wc, stream));
     p.rows = d_rows_ + begin;
     p.work_count = wc;
     last_work_count_ = wc;
@@ -418,11 +384,10 @@ int Engine::launch_range_into(double *d_flux, const double *d_origin, const doub
   if (variant_is_gather(variant)) {
     // counting sort of the range's flying particles by seed-grid cell of their origin
     unsigned int *wc = d_work_count_ + (ticket_next_ % kTicketRing);
-    const double *key = d_origin;  // no origin array (pinned-caller host path): the stored position
     SeedGrid bin_grid = grid_;
     if (!morton_) bin_grid.cell_rank = nullptr;
     p.claim_run = claim_run_;
-    PTB_CUDA_OK(launch_bin_particles(bin_grid, key, d_state_, (bin_midpoint_ && d_dest) ? d_dest : nullptr, d_flying, begin, end, d_pcell_, d_cell_count_,
+    PTB_CUDA_OK(launch_bin_particles(bin_grid, d_origin, d_state_, d_flying, begin, end, d_pcell_, d_cell_count_,
                                      d_cell_sums_, d_order_ + begin, wc, stream));
     p.order = d_order_ + begin;
     p.work_count = wc;
@@ -564,26 +529,11 @@ int Engine::ensure_stage_buffers(const void *caller_mem, size_t caller_bytes) {
   if (posix_memalign(&base, size_t(2) << 20, total) == 0) {
     madvise(base, total, MADV_HUGEPAGE);  // 2 MB pages where the kernel offers them: three streams of TLB misses less
     const int T = pool_->size();
-    // Where the staging slots live.  Default: on the workers' node (= the caller's arrays' node).
-    // PUMITALLY_STAGE_NODE=<n> puts them on another node: on a two-socket host the pass then draws on
-    // both sockets' memory controllers (caller arrays on one, slots + DMA reads on the other).
-    const char *env_node = std::getenv("PUMITALLY_STAGE_NODE");
-    const std::vector<int> there;  // (placement is done with mbind below: the other node's CPUs may not be in the mask)
-    if (env_node) {
-      unsigned long mask[16] = {0};
-      const int node = std::atoi(env_node);
-      if (node >= 0 && node < 1024) {
-        mask[node / 64] = 1ul << (node % 64);
-        if (syscall(SYS_mbind, base, total, 2 /* MPOL_BIND */, mask, 1024ul, 0u) != 0)
-          fprintf(stderr, "[pumitally] WARNING: mbind of the staging slots to node %d failed\n", node);
-      }
-    }
     pool_->run([&](int t) {  // first touch on the workers' NUMA node
       const size_t lo = (total * size_t(t) / size_t(T)) & ~size_t(4095);
       const size_t hi = t == T - 1 ? total : (total * size_t(t + 1) / size_t(T)) & ~size_t(4095);
       std::memset(static_cast<char *>(base) + lo, 0, hi - lo);
     });
-    if (!there.empty() && pool_node_ >= 0) pool_->repin(numa_node_cpus(pool_node_));
     if (cudaHostRegister(base, total, cudaHostRegisterDefault) == cudaSuccess) {
       stage_registered_ = true;
     } else {
@@ -722,13 +672,6 @@ int Engine::move_host(const double *origin, const double *dest, int8_t *flying, 
                       ensure_patch_buffers(nchunks) == 0;
   if (!staged) return move_direct(origin, dest, flying, weights, nchunks);
   follow_caller_memory(dest, size_t(size) * sizeof(double));
-  // Caller arrays that are page-locked (by the caller, or just above) need no copy into the staging
-  // slots: dest and weights go to the device straight from them, and the origins are compared with
-  // the device's own particle positions, which each move sends back (move_pinned).
-  if (pinned_path_ && host_is_pinned(origin) && host_is_pinned(dest) && host_is_pinned(weights) &&
-      ensure_position_mirror(nchunks) == 0)
-    return move_pinned(origin, dest, flying, weights, nchunks);
-  pos_mirror_valid_ = false;  // the move below does not send positions back
 
   // a chunk's staging slots may be refilled once the previous move's copies out of them are done;
   // with an unchanged chunking that is chunk_events_[k], otherwise wait for the whole copy stream
@@ -738,7 +681,6 @@ int Engine::move_host(const double *origin, const double *dest, int8_t *flying, 
   }
   const bool compare = mirror_valid_;
   mirror_valid_ = false;  // until this move has gone through completely
-  stager_->set_buffers(h_dest_, h_w_, h_fly_);
   cudaEvent_t ev_prev_done = chunk_events_[nchunks];
   // the device staging arrays are free once the previous move's kernels have finished
   PTB_CUDA_OK(cudaEventRecord(ev_prev_done, compute_));
@@ -812,147 +754,6 @@ int Engine::move_host(const double *origin, const double *dest, int8_t *flying, 
   return 0;
 }
 
-// Pinned mirror of the particle positions as the device holds them (x,y,z per particle, the layout of
-// the caller's origin array), refreshed by every move of the pinned-caller path.
-int Engine::ensure_position_mirror(int nchunks) {
-  if (!h_pos_) {
-    const size_t bytes = (3 * std::max<size_t>(size_t(n_), 1) * sizeof(double) + 4095) & ~size_t(4095);
-    void *base = nullptr;
-    if (posix_memalign(&base, 4096, bytes) == 0) {
-      HostPool &pool = stager_->pool();
-      const int T = pool.size();
-      pool.run([&](int t) {
-        const size_t lo = (bytes * size_t(t) / size_t(T)) & ~size_t(4095);
-        const size_t hi = t == T - 1 ? bytes : (bytes * size_t(t + 1) / size_t(T)) & ~size_t(4095);
-        std::memset(static_cast<char *>(base) + lo, 0, hi - lo);
-      });
-      if (cudaHostRegister(base, bytes, cudaHostRegisterDefault) != cudaSuccess) {
-        cudaGetLastError();
-        free(base);
-        base = nullptr;
-      }
-    }
-    if (!base) {
-      pinned_path_ = false;  // no pinned memory for the mirror: the staged path serves pinned callers too
-      return 1;
-    }
-    h_pos_ = static_cast<double *>(base);
-    PTB_CUDA_OK(cudaStreamCreateWithFlags(&d2h_, cudaStreamNonBlocking));
-  }
-  while (int(pos_events_.size()) < nchunks) {
-    cudaEvent_t a, b;
-    PTB_CUDA_OK(cudaEventCreateWithFlags(&a, cudaEventDisableTiming));
-    PTB_CUDA_OK(cudaEventCreateWithFlags(&b, cudaEventDisableTiming));
-    pos_events_.push_back(a);
-    walk_events_.push_back(b);
-  }
-  return 0;
-}
-
-// Host-pointer move when the caller's origin / dest / weights arrays are page-locked.
-//
-// Nothing is copied on the host except flying[] (1 byte per particle, so that it can be zeroed at
-// once): dest and weights are DMA'd from the caller's arrays, chunk by chunk.  The origins are not
-// sent at all; the pool compares them with h_pos_, the device's own particle positions as of the end
-// of the previous move (exact bit patterns, hull clip points included), and only particles that fly
-// from somewhere else are listed.  On the device the listed particles are relocated first (phase 1,
-// tally off: relocate_patches), then the walk kernel runs with "origin == stored position" for every
-// particle, then the chunk's new positions are exported and sent back on the otherwise idle
-// device->host direction of the link.  Host memory traffic per particle: 24 B origin + 24 B mirror
-// read by the pool, 33 B read and 24 B written by the DMA engines -- half of the staged path's.
-int Engine::move_pinned(const double *origin, const double *dest, int8_t *flying, const double *weights,
-                        int nchunks) {
-  mirror_valid_ = false;  // the staged path's mirror does not see this move
-  if (!ev_copy0_) {
-    PTB_CUDA_OK(cudaEventCreate(&ev_copy0_));
-    PTB_CUDA_OK(cudaEventCreate(&ev_copy1_));
-  }
-  if (staged_chunk_ != chunk_ || staged_chunks_ != nchunks || !pos_mirror_valid_) {
-    PTB_CUDA_OK(cudaStreamSynchronize(copy_));
-    PTB_CUDA_OK(cudaStreamSynchronize(d2h_));
-    staged_chunks_ = 0;
-  }
-  if (!pos_mirror_valid_) {  // first move on this path, or moves in between that sent nothing back
-    PTB_CUDA_OK(launch_export_positions(d_state_, d_origin_, 0, n_, compute_));
-    PTB_CUDA_OK(cudaMemcpyAsync(h_pos_, d_origin_, 3 * size_t(n_) * sizeof(double), cudaMemcpyDeviceToHost, compute_));
-    PTB_CUDA_OK(cudaStreamSynchronize(compute_));
-    ++launches_;
-  }
-  pos_mirror_valid_ = false;  // until this move has gone through completely
-  stager_->set_buffers(nullptr, nullptr, h_fly_, h_pos_);
-  cudaEvent_t ev_prev_done = chunk_events_[nchunks];
-  PTB_CUDA_OK(cudaEventRecord(ev_prev_done, compute_));
-  PTB_CUDA_OK(cudaStreamWaitEvent(copy_, ev_prev_done, 0));
-  double sent = 0.0;
-  const auto t_begin = std::chrono::steady_clock::now();
-  auto range_of = [&](int k, int32_t &b, int32_t &e) {
-    b = int32_t(int64_t(k) * chunk_);
-    e = int32_t(std::min<int64_t>(n_, int64_t(b) + chunk_));
-  };
-  auto start_stage = [&](int k) -> int {
-    if (k < staged_chunks_) {
-      PTB_CUDA_OK(cudaEventSynchronize(chunk_events_[k]));  // previous move's upload of the chunk's flying slots
-      PTB_CUDA_OK(cudaEventSynchronize(pos_events_[k]));    // its positions are back
-    }
-    if (k >= kPatchSlots) PTB_CUDA_OK(cudaEventSynchronize(chunk_events_[k - kPatchSlots]));
-    int32_t b, e;
-    range_of(k, b, e);
-    stager_->begin(origin, dest, flying, weights, b, e, true, h_patch_ + size_t(k % kPatchSlots) * patch_cap_);
-    return 0;
-  };
-  PTB_CUDA_OK(cudaEventRecord(ev_copy0_, copy_));
-  if (nchunks > 0 && start_stage(0)) return 1;
-  for (int k = 0; k < nchunks; ++k) {
-    int32_t b, e;
-    range_of(k, b, e);
-    const size_t cnt = size_t(e - b);
-    const int64_t npatch = stager_->end();
-    if (k + 1 < nchunks && start_stage(k + 1)) return 1;
-    PatchEntry *hp = h_patch_ + size_t(k % kPatchSlots) * patch_cap_, *dp = d_patch_ + size_t(k) * patch_cap_;
-    PTB_CUDA_OK(cudaMemcpyAsync(d_flying_ + b, h_fly_ + b, cnt, cudaMemcpyHostToDevice, copy_));
-    if (npatch < 0) {  // most of the chunk was re-sourced: its origins travel whole, the kernel sorts them out
-      PTB_CUDA_OK(cudaStreamWaitEvent(copy_, walk_events_[k], 0));  // d_origin_ doubles as the export buffer
-      PTB_CUDA_OK(cudaMemcpyAsync(d_origin_ + 3 * size_t(b), origin + 3 * size_t(b), 3 * cnt * sizeof(double), cudaMemcpyHostToDevice, copy_));
-      sent += 24.0 * double(cnt);
-    } else if (npatch > 0) {
-      PTB_CUDA_OK(cudaMemcpyAsync(dp, hp, size_t(npatch) * sizeof(PatchEntry), cudaMemcpyHostToDevice, copy_));
-      sent += double(npatch) * sizeof(PatchEntry);
-    }
-    PTB_CUDA_OK(cudaMemcpyAsync(d_dest_ + 3 * size_t(b), dest + 3 * size_t(b), 3 * cnt * sizeof(double), cudaMemcpyHostToDevice, copy_));
-    PTB_CUDA_OK(cudaMemcpyAsync(d_weights_ + b, weights + b, cnt * sizeof(double), cudaMemcpyHostToDevice, copy_));
-    sent += 33.0 * double(cnt);
-    PTB_CUDA_OK(cudaEventRecord(chunk_events_[k], copy_));
-    PTB_CUDA_OK(cudaStreamWaitEvent(compute_, chunk_events_[k], 0));
-    // the export below reuses d_origin_: the previous move's device->host copy out of it must be done
-    PTB_CUDA_OK(cudaStreamWaitEvent(compute_, pos_events_[k], 0));
-    if (npatch > 0 && relocate_patches(dp, int32_t(npatch), compute_)) return 1;
-    if (launch_range(npatch < 0 ? d_origin_ : nullptr, d_dest_, d_flying_, d_weights_, b, e, compute_, true)) return 1;
-    PTB_CUDA_OK(launch_export_positions(d_state_, d_origin_, b, e, compute_));
-    ++launches_;
-    PTB_CUDA_OK(cudaEventRecord(walk_events_[k], compute_));
-    PTB_CUDA_OK(cudaStreamWaitEvent(d2h_, walk_events_[k], 0));
-    static const bool debug_no_d2h = std::getenv("PUMITALLY_DEBUG_NO_D2H") != nullptr;  // timing experiments only: wrong results
-    if (!debug_no_d2h)
-    PTB_CUDA_OK(cudaMemcpyAsync(h_pos_ + 3 * size_t(b), d_origin_ + 3 * size_t(b), 3 * cnt * sizeof(double), cudaMemcpyDeviceToHost, d2h_));
-    PTB_CUDA_OK(cudaEventRecord(pos_events_[k], d2h_));
-  }
-  PTB_CUDA_OK(cudaEventRecord(ev_copy1_, copy_));
-  if (mark_move_done()) return 1;
-  // dest and weights are read from the caller's own arrays: they must be on the device before the
-  // caller gets them back (reference: blocking deep_copy)
-  PTB_CUDA_OK(cudaStreamSynchronize(copy_));
-  stage_host_s_ = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_begin).count();
-  stage_sent_bytes_ = sent;
-  h2d_bytes_ += sent;
-  d2h_bytes_ += 24.0 * double(n_);
-  staged_chunk_ = chunk_;
-  staged_chunks_ = nchunks;
-  pos_mirror_valid_ = true;
-  initial_weight_pending_ = false;
-  ++moves_;
-  return 0;
-}
-
 // Device time the previous host move's uploads took (first copy could start -> last copy done), credited to
 // the path that move used; feeds the staged-vs-direct choice for page-locked caller arrays.
 void Engine::collect_upload_span() {
@@ -982,7 +783,6 @@ int Engine::mark_move_done() {
 int Engine::move_direct(const double *origin, const double *dest, int8_t *flying, const double *weights,
                         int nchunks) {
   mirror_valid_ = false;  // the staging slots do not see this move
-  pos_mirror_valid_ = false;
   cudaEvent_t ev_prev_done = chunk_events_[nchunks], ev_fly = chunk_events_[nchunks + 1];
   PTB_CUDA_OK(cudaStreamSynchronize(copy_));  // staged copies of an earlier move
   staged_chunks_ = 0;
@@ -1029,9 +829,7 @@ int Engine::move_to_next_location_device(const double *d_origin, const double *d
   PTB_CUDA_OK(cudaSetDevice(device_));
   begin_move();
   // (the staging arrays are not touched: "pinned dest slots == device dest array" keeps holding, and the
-  // next host move's origins are compared against them and patched exactly as after a host move;
-  // the position mirror of the pinned-caller path, however, is out of date after this move)
-  pos_mirror_valid_ = false;
+  // next host move's origins are compared against them and patched exactly as after a host move)
   if (launch_range(d_origin, d_dest, d_flying, d_weights, 0, n_, stream, true)) return 1;
   initial_weight_pending_ = false;
   ++moves_;
@@ -1063,7 +861,7 @@ int Engine::set_score_bins(int32_t nbins) {
 
 // MoveToNextLocation with a score bin per particle for this move (host pointers).  bins == nullptr or one
 // bin: the plain move.  The bins travel in one copy ahead of the particle data; everything else is the
-// ordinary host path (the pinned-caller variant excepted, whose relocation pass knows nothing of bins).
+// ordinary host path.
 int Engine::move_to_next_location_binned(const double *origin, const double *dest, int8_t *flying, const double *weights,
                                          const int32_t *bins, int32_t size) {
   if (!bins || nbins_ == 1) return move_to_next_location(origin, dest, flying, weights, size);
@@ -1105,15 +903,12 @@ int Engine::move_to_next_location_binned(const double *origin, const double *des
   PTB_CUDA_OK(cudaEventRecord(ev_bins_, copy_));
   h2d_bytes_ += 4.0 * double(n_);
   cur_bins_ = d_bins_;
-  const bool pinned_path = pinned_path_;
-  pinned_path_ = false;
   // every pipeline stage is walked nbins + 1 times, seven small launches each, all enqueued by this thread between
   // two stage passes: unless the caller chose the stage size, binned moves use stages of 2 Mi particles
   const int32_t chunk = chunk_;
   if (!chunk_user_set_) chunk_ = std::max(chunk_, int32_t(1) << 21);
   const int rc = move_to_next_location(origin, dest, flying, weights, size);
   chunk_ = chunk;
-  pinned_path_ = pinned_path;
   cur_bins_ = nullptr;
   PTB_CUDA_OK(cudaEventSynchronize(ev_bins_));  // the caller gets `bins` back with the other arrays
   return rc;
@@ -1154,7 +949,6 @@ int Engine::set_state_device(const double *d_xyz, const int32_t *d_elem, int32_t
   PTB_CUDA_OK(launch_set_state(d_state_, d_xyz, d_elem, d_internal_of_orig_, first, first + count, stream));
   initialized_ = true;
   mirror_valid_ = false;
-  pos_mirror_valid_ = false;
   return 0;
 }
 
@@ -1309,7 +1103,6 @@ int64_t Engine::get_option(const std::string &name) const {
   if (name == "seed_grid") return seed_grid_mode_;
   if (name == "seed_grid_active") return use_seed_grid_ ? 1 : 0;
   if (name == "hull_convex") return mesh_.hull_convex ? 1 : 0;
-  if (name == "bin_midpoint") return bin_midpoint_ ? 1 : 0;
   if (name == "max_iters") return max_iters_;
   if (name == "l2_fetch") {
     size_t g = 0;
@@ -1317,16 +1110,11 @@ int64_t Engine::get_option(const std::string &name) const {
   }
   if (name == "allreduce_us") return int64_t(allreduce_ms_ * 1e3);  // device time of the last batch-end exchange
   if (name == "score_bins") return nbins_;
-  if (name == "die_split") return die_split_ ? 1 : 0;
-  if (name == "l2_partition0_sms") return die0_sms_;  // SMs in the L2 partition of SM 0 (0: no map found)
   if (name == "exchange_choice") return exchange_choice_;  // what exchange_tally() does: 0 all-reduce, 1 reduce-scatter
   if (name == "exchange_allreduce_us") return int64_t(exchange_ms_[0] * 1e3);  // comm_init's measurement of the two
   if (name == "exchange_reduce_scatter_us") return int64_t(exchange_ms_[1] * 1e3);
-  if (name == "d2h_bytes") return int64_t(d2h_bytes_);  // particle positions sent back by the pinned-caller path, cumulative
   if (name == "host_path") return host_path_;
   if (name == "host_path_last") return span_tag_ == 1 ? 0 : 1;  // path of the last host move: 1 staged, 0 direct
-  if (name == "pinned_path") return pinned_path_ ? 1 : 0;
-  if (name == "position_mirror") return pos_mirror_valid_ ? 1 : 0;  // the last host move took the pinned-caller path
   if (name == "host_threads") return stager_ ? stager_->threads() : host_threads_;
   if (name == "stage_host_us") return int64_t(stage_host_s_ * 1e6);   // last staged move: host time from entry to return
   if (name == "stage_sent_bytes") return int64_t(stage_sent_bytes_);  // last staged move: bytes put on the wire
@@ -1371,27 +1159,6 @@ int Engine::set_option(const std::string &name, int64_t v) {
     if (v < 1024) return 1;
     chunk_ = int32_t(std::min<int64_t>(v, INT_MAX)) & ~1023;  // keeps every range 16-byte aligned
     chunk_user_set_ = true;
-  } else if (name == "die_split") {
-    // Experiment, off by default (measured: c4 5 % slower, c5 1.6 % faster, c2 unchanged -- profiles/r02/README.md):
-    // the SMs of each L2 partition take the sorted particles from their own end of the sequence.
-    die_split_ = v != 0;
-    if (die_split_) {
-      // which SMs share an L2 partition: probed once per device and process (a few ms)
-      struct Cached { bool done = false; uint32_t mask[8]; int die0 = 0, nsms = 0; };
-      static Cached cache[64];
-      static std::mutex cache_mutex;
-      std::lock_guard<std::mutex> lock(cache_mutex);
-      Cached &c = cache[device_ & 63];
-      if (!c.done) {
-        PTB_CUDA_OK(cudaSetDevice(device_));
-        PTB_CUDA_OK(cudaDeviceSynchronize());
-        if (probe_l2_partitions(c.mask, &c.die0, &c.nsms, compute_) != 0) c.die0 = 0;
-        c.done = true;
-      }
-      for (int i = 0; i < 8; ++i) die_mask_[i] = c.mask[i];
-      die0_sms_ = c.die0;
-      nsms_ = c.nsms;
-    }
   } else if (name == "exchange_choice") {
     exchange_choice_ = v ? 1 : 0;  // the caller must set the same value on every rank
   } else if (name == "seed_grid") {
@@ -1410,13 +1177,9 @@ int Engine::set_option(const std::string &name, int64_t v) {
     if (v < 0 || v > 2) return 1;
     host_path_ = int(v);
     if (host_path_ == 0) mirror_valid_ = false;
-  } else if (name == "pinned_path") {  // 0 = page-locked caller arrays also go through the staging slots
-    pinned_path_ = v != 0;
   } else if (name == "host_threads") {  // workers of the staging pool; before the first host-pointer call
     if (v < 1 || v > 256 || stager_) return 1;
     host_threads_ = int(v);
-  } else if (name == "bin_midpoint") {  // binning key: cell of the track's midpoint instead of its start
-    bin_midpoint_ = v != 0;
   } else if (name == "morton") {
     morton_ = v != 0;
   } else if (name == "claim_run") {

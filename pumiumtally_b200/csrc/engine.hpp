@@ -98,10 +98,6 @@ class Engine {
   int move_host(const double *origin, const double *dest, int8_t *flying, const double *weights, int32_t size);
   int launch_range_into(double *d_flux, const double *d_origin, const double *d_dest, const int8_t *d_flying,
                         const double *d_weights, int32_t begin, int32_t end, cudaStream_t stream, bool timed);
-  // L2 partition of every SM (l2_partitions.cu), probed when option die_split is switched on; die0_sms_ == 0: no usable map
-  uint32_t die_mask_[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-  int die0_sms_ = 0, nsms_ = 0;
-  bool die_split_ = false;
   int32_t nbins_ = 1;
   size_t flux_alloc_ = 0;             // doubles allocated at d_flux_
   size_t flux_len() const { return size_t(nbins_) * size_t(mesh_.ntets); }  // reported part of d_flux_
@@ -153,7 +149,6 @@ class Engine {
   int32_t max_iters_ = 0;  // crossing limit per walk; 0 = ntets + 16
   bool morton_ = true;    // binning key: Morton rank of the cell (matches the tet storage order) instead of its z-major index
   int claim_run_ = 4;     // chunks per ticket in gather mode
-  bool bin_midpoint_ = false;  // binning key: cell of the track's midpoint instead of its start (experiment, c5)
 
   // device memory
   TetRecord *d_tets_ = nullptr;
@@ -228,18 +223,6 @@ class Engine {
   void follow_caller_memory(const void *p, size_t bytes);
   int ensure_patch_buffers(int nchunks);
   int move_direct(const double *origin, const double *dest, int8_t *flying, const double *weights, int nchunks);
-  // Page-locked caller arrays (pinned by the caller, or by option register_host): see move_pinned().
-  // Off by default: on the measured box the positions travelling back (24 B per particle, device->host)
-  // slow the uploads down more than the saved host work buys (profiles/r02/README.md).
-  bool pinned_path_ = false;
-  double *h_pos_ = nullptr;            // pinned mirror of the device's particle positions [3N]
-  bool pos_mirror_valid_ = false;
-  cudaStream_t d2h_ = nullptr;
-  std::vector<cudaEvent_t> pos_events_, walk_events_;  // per chunk: positions back on the host / walk + export done
-  double d2h_bytes_ = 0.0;
-  int ensure_position_mirror(int nchunks);
-  int move_pinned(const double *origin, const double *dest, int8_t *flying, const double *weights, int nchunks);
-  int relocate_patches(const PatchEntry *d_list, int32_t count, cudaStream_t stream);
 
   // NCCL (resolved with dlopen at comm_init time)
   void *nccl_comm_ = nullptr;

@@ -254,27 +254,24 @@ inline void record(const double *o, int64_t i, PatchEntry *patches, int64_t &np,
   ++np;
 }
 
-inline void stage_one(const double *origin, const double *dest, const double *weights, const double *mirror,
-                      double *b_dest, double *b_w, int64_t i, bool compare, PatchEntry *patches, int64_t &np,
-                      int64_t cap) {
-  if (compare && differs(origin + 3 * i, mirror + 3 * i)) record(origin + 3 * i, i, patches, np, cap);
-  if (b_dest) {
-    b_dest[3 * i] = dest[3 * i];
-    b_dest[3 * i + 1] = dest[3 * i + 1];
-    b_dest[3 * i + 2] = dest[3 * i + 2];
-    b_w[i] = weights[i];
-  }
+inline void stage_one(const double *origin, const double *dest, const double *weights, double *b_dest, double *b_w,
+                      int64_t i, bool compare, PatchEntry *patches, int64_t &np, int64_t cap) {
+  if (compare && differs(origin + 3 * i, b_dest + 3 * i)) record(origin + 3 * i, i, patches, np, cap);
+  b_dest[3 * i] = dest[3 * i];
+  b_dest[3 * i + 1] = dest[3 * i + 1];
+  b_dest[3 * i + 2] = dest[3 * i + 2];
+  b_w[i] = weights[i];
 }
 
-int64_t stage_scalar(const double *origin, const double *dest, int8_t *flying, const double *weights,
-                     const double *mirror, double *b_dest, double *b_w, int8_t *b_fly, int64_t lo, int64_t hi,
-                     bool compare, PatchEntry *patches, int64_t cap) {
+int64_t stage_scalar(const double *origin, const double *dest, int8_t *flying, const double *weights, double *b_dest,
+                     double *b_w, int8_t *b_fly, int64_t lo, int64_t hi, bool compare, PatchEntry *patches,
+                     int64_t cap) {
   int64_t np = 0;
   for (int64_t i = lo; i < hi; ++i) {
     const int8_t f = flying[i];
     b_fly[i] = f;
     flying[i] = 0;
-    stage_one(origin, dest, weights, mirror, b_dest, b_w, i, compare && f == 1, patches, np, cap);
+    stage_one(origin, dest, weights, b_dest, b_w, i, compare && f == 1, patches, np, cap);
   }
   return np <= cap ? np : -1;
 }
@@ -300,15 +297,15 @@ __attribute__((target("avx2"))) void copy_block(double *dst, const double *src, 
 }
 
 __attribute__((target("avx2"))) int64_t stage_avx2(const double *origin, const double *dest, int8_t *flying,
-                                                   const double *weights, const double *mirror, double *b_dest,
-                                                   double *b_w, int8_t *b_fly, int64_t lo, int64_t hi, bool compare,
-                                                   PatchEntry *patches, int64_t cap) {
+                                                   const double *weights, double *b_dest, double *b_w, int8_t *b_fly,
+                                                   int64_t lo, int64_t hi, bool compare, PatchEntry *patches,
+                                                   int64_t cap) {
   int64_t np = 0;
   for (int64_t b0 = lo; b0 < hi; b0 += kBlock) {
     const int64_t b1 = std::min(hi, b0 + kBlock), cnt = b1 - b0;
     if (compare) {
       const double *o = origin + 3 * b0;
-      const double *m = mirror + 3 * b0;
+      const double *m = b_dest + 3 * b0;
       int64_t g = 0;
       for (; g + 4 <= cnt; g += 4) {  // 4 particles = 96 bytes = three 256-bit lanes
         const double *og = o + 3 * g, *mg = m + 3 * g;
@@ -324,9 +321,8 @@ __attribute__((target("avx2"))) int64_t stage_avx2(const double *origin, const d
       for (; g < cnt; ++g)
         if (flying[b0 + g] == 1 && differs(o + 3 * g, m + 3 * g)) record(o + 3 * g, b0 + g, patches, np, cap);
     }
-    if (b_dest) copy_block(b_dest + 3 * b0, dest + 3 * b0, 3 * cnt);
-    if (!b_w) {
-    } else if (cnt == kBlock && (reinterpret_cast<uintptr_t>(b_w + b0) & 63u) == 0) {
+    copy_block(b_dest + 3 * b0, dest + 3 * b0, 3 * cnt);
+    if (cnt == kBlock && (reinterpret_cast<uintptr_t>(b_w + b0) & 63u) == 0) {
       // the weight slots are written only: whole 64-byte lines with non-temporal stores, no
       // read-for-ownership (the dest slots above were just read by the compare pass)
       for (int64_t k = 0; k < kBlock; k += 8) {
@@ -347,13 +343,13 @@ __attribute__((target("avx2"))) int64_t stage_avx2(const double *origin, const d
 }  // namespace
 
 int64_t stage_range(const double *origin, const double *dest, int8_t *flying, const double *weights,
-                    const double *mirror, double *b_dest, double *b_w, int8_t *b_fly, int64_t lo, int64_t hi,
-                    bool compare, PatchEntry *patches, int64_t cap) {
+                    double *b_dest, double *b_w, int8_t *b_fly, int64_t lo, int64_t hi, bool compare,
+                    PatchEntry *patches, int64_t cap) {
   static const bool have_avx2 = __builtin_cpu_supports("avx2");
   static const bool force_scalar = std::getenv("PUMITALLY_STAGE_SCALAR") != nullptr;
   if (have_avx2 && !force_scalar)
-    return stage_avx2(origin, dest, flying, weights, mirror, b_dest, b_w, b_fly, lo, hi, compare, patches, cap);
-  return stage_scalar(origin, dest, flying, weights, mirror, b_dest, b_w, b_fly, lo, hi, compare, patches, cap);
+    return stage_avx2(origin, dest, flying, weights, b_dest, b_w, b_fly, lo, hi, compare, patches, cap);
+  return stage_scalar(origin, dest, flying, weights, b_dest, b_w, b_fly, lo, hi, compare, patches, cap);
 }
 
 // ------------------------------------------------------------------------------- stager
@@ -396,8 +392,8 @@ void HostStager::work(int t) {
     const int64_t lo = j.b + blk * kGrain;
     if (lo >= j.e) break;
     const int64_t hi = std::min(j.e, lo + kGrain);
-    const int64_t c = stage_range(j.origin, j.dest, j.flying, j.weights, mirror_, b_dest_, b_w_, b_fly_, lo, hi,
-                                  j.compare, mine + np, int64_t(tls_cap_) - np);
+    const int64_t c = stage_range(j.origin, j.dest, j.flying, j.weights, b_dest_, b_w_, b_fly_, lo, hi, j.compare,
+                                  mine + np, int64_t(tls_cap_) - np);
     if (c < 0) overflow = true;
     else np += c;
   }

@@ -86,12 +86,9 @@ std::vector<int> numa_node_cpus(int node);
 // flight merely reports its origin as changed, and the device decides exactly as always.)
 // Returns the number of patch entries written, or -1 if they did not fit in `cap` (the range is
 // staged completely either way).
-// `mirror` is what the origins are compared against: b_dest itself in the staged path, the device's
-// exported particle positions in the pinned-caller path, where b_dest and b_w are null (dest and
-// weights then go to the device straight from the caller's pinned arrays and are not copied here).
 int64_t stage_range(const double *origin, const double *dest, int8_t *flying, const double *weights,
-                    const double *mirror, double *b_dest, double *b_w, int8_t *b_fly, int64_t lo, int64_t hi,
-                    bool compare, PatchEntry *patches, int64_t cap);
+                    double *b_dest, double *b_w, int8_t *b_fly, int64_t lo, int64_t hi, bool compare,
+                    PatchEntry *patches, int64_t cap);
 
 
 // One chunk of a move at a time: the pool's workers split particles [b, e), run stage_range on their
@@ -104,9 +101,8 @@ class HostStager {
   }
   int threads() const { return pool_.size(); }
   HostPool &pool() { return pool_; }
-  // mirror == nullptr: the dest slots are the mirror
-  void set_buffers(double *b_dest, double *b_w, int8_t *b_fly, const double *mirror = nullptr) {
-    b_dest_ = b_dest; b_w_ = b_w; b_fly_ = b_fly; mirror_ = mirror ? mirror : b_dest;
+  void set_buffers(double *b_dest, double *b_w, int8_t *b_fly) {
+    b_dest_ = b_dest; b_w_ = b_w; b_fly_ = b_fly;
   }
   void reserve(size_t cap);  // largest list a chunk may produce
   void begin(const double *origin, const double *dest, int8_t *flying, const double *weights, int64_t b,
@@ -118,7 +114,6 @@ class HostStager {
   HostPool pool_;
   std::function<void(int)> fn_;
   double *b_dest_ = nullptr, *b_w_ = nullptr;
-  const double *mirror_ = nullptr;
   int8_t *b_fly_ = nullptr;
   static constexpr int64_t kGrain = 2048;  // particles per claimed block (multiple of the pass's 256-particle tile)
   std::atomic<int64_t> next_block_{0};

@@ -300,12 +300,6 @@ struct WalkParams {
   DeviceStats *stats;
   SeedGrid grid;
   double cx, cy, cz;           // mesh centre: the planes are stored relative to it (tet_mesh.hpp)
-  // Sorted (gather / packed) modes, optional: the SMs of each L2 partition work on their own end of the sorted
-  // particle sequence (walk_persist.cuh, "die split").  die_mask bit s = partition of SM s; die0_sms of nsms SMs
-  // are in partition 0; work_counter2 is the second partition's chunk ticket.  die0_sms == 0: off.
-  uint32_t die_mask[8];
-  int32_t die0_sms, nsms;
-  unsigned int *work_counter2;
 };
 
 constexpr int kStageReloc = 0;  // phase 1: move to caller's origin, tally off

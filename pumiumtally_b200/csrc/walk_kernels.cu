@@ -90,41 +90,6 @@ __global__ void patch_origins_kernel(double *origin, const PatchEntry *list, int
   origin[3 * (size_t)idx + 2] = z;
 }
 
-// Relocation of re-sourced particles ahead of the walk kernel (launch_relocate_patches): thread per
-// entry, the same state machine as walk_ldg_kernel with the tally phase switched off.
-__global__ void __launch_bounds__(128) relocate_patches_kernel(WalkParams P, const PatchEntry *list, int32_t count,
-                                                               int8_t *flying) {
-  const int k = blockIdx.x * blockDim.x + threadIdx.x;
-  Counters c;
-  Ray r;
-  r.stage = kStageDone;
-  int i = 0;
-  if (k < count) {
-    double tx, ty, tz, tail;
-    load_face_256(reinterpret_cast<const double *>(list + k), tx, ty, tz, tail);
-    i = (int32_t)((unsigned long long)__double_as_longlong(tail) & 0xffffffffull);
-    const ParticleState s0 = load_state(P.state + i);
-    r.e = s0.elem;
-    if (!all_finite(tx, ty, tz)) {  // unusable origin: the particle sits this move out
-      flying[i] = 0;
-      c.lost++;
-    } else if (tx != s0.x || ty != s0.y || tz != s0.z) {
-      start_reloc(P, r, s0.x, s0.y, s0.z, tx, ty, tz);
-    }
-  }
-  while (r.stage != kStageDone) {
-    const double *rec = P.tets[r.e].d;
-    double raw[16];
-#pragma unroll
-    for (int f = 0; f < 4; ++f)
-      load_face_256(rec + 4 * f, raw[4 * f], raw[4 * f + 1], raw[4 * f + 2], raw[4 * f + 3]);
-    ExitScan sc;
-    scan_record(raw, r.e, r.ox, r.oy, r.oz, r.ux, r.uy, r.uz, sc);
-    advance(P, i, r, exit_parameter(sc), sc.nbr, sc.back, c, true);
-  }
-  flush_counters(P, c);
-}
-
 // Particle slots [begin, end) <- (xyz, element in the caller's numbering): for callers that manage
 // particle placement themselves (the spatially partitioned multi-GPU driver hands particles from one
 // picpart to the next).  elem_map: caller's element id -> internal id.
@@ -153,15 +118,6 @@ __global__ void get_state_kernel(const ParticleState *state, double *xyz, int32_
 __global__ void flux_to_caller_order_kernel(const double *flux, const int32_t *orig_of_internal, double *out, int64_t n) {
   const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (e < n) out[orig_of_internal[e]] = flux[e];
-}
-
-__global__ void export_positions_kernel(const ParticleState *state, double *xyz, int32_t begin, int32_t end) {
-  const int i = begin + blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= end) return;
-  const ParticleState s = load_state(state + i);
-  xyz[3 * (size_t)i] = s.x;
-  xyz[3 * (size_t)i + 1] = s.y;
-  xyz[3 * (size_t)i + 2] = s.z;
 }
 
 // K13 (PumiTallyImpl.cpp:393-405) with volumes precomputed at mesh build.
@@ -262,18 +218,6 @@ cudaError_t launch_patch_origins(double *origin, const PatchEntry *list, int32_t
   return cudaGetLastError();
 }
 
-cudaError_t launch_relocate_patches(const WalkParams &p, const PatchEntry *list, int32_t count, int8_t *flying,
-                                    cudaStream_t stream) {
-  if (count <= 0) return cudaSuccess;
-  WalkParams q = p;
-  q.origin = nullptr;  // unused: the targets come from the list
-  q.dest = nullptr;    // end_ray() stores the state when phase 1 ends
-  q.weights = nullptr;
-  q.flying = nullptr;
-  relocate_patches_kernel<<<(count + 127) / 128, 128, 0, stream>>>(q, list, count, flying);
-  return cudaGetLastError();
-}
-
 cudaError_t launch_set_state(ParticleState *state, const double *xyz, const int32_t *elem, const int32_t *elem_map,
                              int32_t begin, int32_t end, cudaStream_t stream) {
   if (end <= begin) return cudaSuccess;
@@ -292,13 +236,6 @@ cudaError_t launch_flux_to_caller_order(const double *flux, const int32_t *orig_
                                         cudaStream_t stream) {
   if (n <= 0) return cudaSuccess;
   flux_to_caller_order_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(flux, orig_of_internal, out, n);
-  return cudaGetLastError();
-}
-
-cudaError_t launch_export_positions(const ParticleState *state, double *xyz, int32_t begin, int32_t end,
-                                    cudaStream_t stream) {
-  if (end <= begin) return cudaSuccess;
-  export_positions_kernel<<<(end - begin + 255) / 256, 256, 0, stream>>>(state, xyz, begin, end);
   return cudaGetLastError();
 }
 

@@ -57,9 +57,8 @@ inline bool variant_is_packed(int v) {
 cudaError_t launch_walk(const WalkParams &p, int variant, int block, cudaStream_t stream);
 bool walk_variant_available(int variant);  // compiled into this library?
 // origin == nullptr: the binning key is the stored position (state)
-// mid != nullptr: the key is the midpoint of (start, mid[i]) -- pass the dest array
 cudaError_t launch_bin_particles(const SeedGrid &g, const double *origin, const ParticleState *state,
-                                 const double *mid, const int8_t *flying, int32_t begin, int32_t end, int32_t *pcell, unsigned int *count,
+                                 const int8_t *flying, int32_t begin, int32_t end, int32_t *pcell, unsigned int *count,
                                  unsigned int *sums, int32_t *order, unsigned int *work_count,
                                  cudaStream_t stream);
 // Like launch_bin_particles, but instead of the id list the scatter pass writes one PackedRow per
@@ -68,7 +67,7 @@ cudaError_t launch_bin_pack_particles(const SeedGrid &g, const double *origin, c
                                       const double *weights, const int8_t *flying, const ParticleState *state,
                                       int32_t begin, int32_t end, int32_t *pcell, unsigned int *count,
                                       unsigned int *sums, PackedRow *rows, unsigned int *work_count,
-                                      bool midpoint_key, cudaStream_t stream);
+                                      cudaStream_t stream);
 cudaError_t launch_seed_points(const SeedGrid &g, double *xyz, cudaStream_t stream);
 cudaError_t launch_seed_finalize(const double *xyz, const ParticleState *state, int32_t *cell_tet,
                                  int32_t ncell, cudaStream_t stream);
@@ -76,13 +75,6 @@ cudaError_t launch_init_particles(ParticleState *state, int32_t n, double cx, do
                                   int32_t elem, cudaStream_t stream);
 // origin[3*idx..] = (x,y,z) for every entry of the patch list
 cudaError_t launch_patch_origins(double *origin, const PatchEntry *list, int32_t count, cudaStream_t stream);
-// Phase 1 of MoveToNextLocation (PumiTallyImpl.cpp:71-112) for the listed particles only: each is
-// walked, tally off, from its stored position to (x,y,z) of its entry and its state is updated; an
-// entry with a non-finite position makes the particle sit the move out (flying[idx] <- 0, counted as
-// lost).  p.origin / p.dest / p.weights are ignored.  For the host path whose mirror is the device's
-// own particle positions: every particle not listed is already where its origin says.
-cudaError_t launch_relocate_patches(const WalkParams &p, const PatchEntry *list, int32_t count, int8_t *flying,
-                                    cudaStream_t stream);
 // particle slots [begin, end) <-> (xyz[3k..], elem[k]) with k = slot - begin; elem in the caller's numbering
 cudaError_t launch_set_state(ParticleState *state, const double *xyz, const int32_t *elem, const int32_t *elem_map,
                              int32_t begin, int32_t end, cudaStream_t stream);
@@ -90,19 +82,14 @@ cudaError_t launch_get_state(const ParticleState *state, double *xyz, int32_t *e
                              int32_t begin, int32_t end, cudaStream_t stream);
 cudaError_t launch_flux_to_caller_order(const double *flux, const int32_t *orig_of_internal, double *out, int64_t n,
                                         cudaStream_t stream);
-// xyz[3i..3i+2] = position of particle i for i in [begin, end)
-cudaError_t launch_export_positions(const ParticleState *state, double *xyz, int32_t begin, int32_t end,
-                                    cudaStream_t stream);
 // out = flux / volume / per_source (NormalizeFlux, PumiTallyImpl.cpp:393-405; per_source = 1 is the reference)
 cudaError_t launch_normalize(const double *flux, const double *volume, double *out, int64_t n,
                              double per_source, cudaStream_t stream);
-// *total += sum of weights[i] over flying particles of [begin, end)
-// l2_partitions.cu: which SMs share an L2 partition (mask bit s = partition of SM s); 0 = found two clear groups
-int probe_l2_partitions(uint32_t mask[8], int *die0_sms, int *nsms, cudaStream_t stream);
 
 // mask[i] = flying[i] && bins[i] == bin  (bin == nbins selects the particles outside [0, nbins))
 cudaError_t launch_bin_mask(const int8_t *flying, const int32_t *bins, int32_t bin, int32_t nbins, int8_t *mask,
                             int32_t begin, int32_t end, cudaStream_t stream);
+// *total += sum of weights[i] over flying particles of [begin, end)
 cudaError_t launch_sum_flying_weights(const int8_t *flying, const double *weights, int32_t begin, int32_t end,
                                       double *total, cudaStream_t stream);
 

@@ -545,51 +545,9 @@ __global__ void __launch_bounds__(BLOCK, MINB) walk_persist_kernel(const WalkPar
   const int claim_run = GATHER ? min(max(P.claim_run, 1), kClaimRun) : 1;
   int run_base = 0, run_next = 0, run_end = 0, ids0 = 0, ids1 = 0;
   int pend_base = -1, pend0 = 0, pend1 = 0;
-  // Die split (sorted modes only).  A B200's L2 is two partitions, one per die, and each keeps its own copy of
-  // every line its SMs touch (profiles/r02/z_l2_probe_die_map.txt: a line only the other die has read costs 467
-  // cycles instead of 290, and a table read by all SMs stays resident only up to half the L2).  When all SMs
-  // work through the sorted particles front to back, both partitions hold the same window of the mesh.  Here
-  // the SMs of partition 0 take chunks from the front of the sequence and those of partition 1 from its own
-  // start further back (the sequence is cut in proportion to the SM counts), so each partition caches only its
-  // own window; a partition that runs out of chunks helps the other finish.
-  constexpr bool kSplit = GATHER || PACKED;
-  constexpr int kNoChunk = 0x3fffffff;
-  int split_phase = 2, own_lo = 0, own_hi = 0, oth_lo = 0, oth_hi = 0;
-  unsigned int *own_cnt = P.work_counter, *oth_cnt = P.work_counter;
-  if constexpr (kSplit) {
-    if (P.die0_sms > 0 && P.die0_sms < P.nsms) {
-      unsigned sm;
-      asm("mov.u32 %0, %%smid;" : "=r"(sm));
-      const int die = (P.die_mask[(sm >> 5) & 7] >> (sm & 31)) & 1;
-      const int mid = (int)((long long)nchunks * P.die0_sms / P.nsms) & ~(kClaimRun - 1);  // tickets never straddle it
-      own_lo = die ? mid : 0; own_hi = die ? nchunks : mid;
-      oth_lo = die ? 0 : mid; oth_hi = die ? mid : nchunks;
-      own_cnt = die ? P.work_counter2 : P.work_counter;
-      oth_cnt = die ? P.work_counter : P.work_counter2;
-      split_phase = 0;
-    }
-  }
   // next ticket of `run` chunks: its first chunk, or a value >= nchunks when nothing is left (warp-uniform)
   auto take = [&](int run) -> int {
     int c = 0;
-    if constexpr (kSplit) {
-      if (split_phase < 2) {
-        if (lane == 0) {
-          c = kNoChunk;
-          if (split_phase == 0) {
-            c = own_lo + (int)atomicAdd(own_cnt, (unsigned)run);
-            if (c >= own_hi) { c = kNoChunk; split_phase = 1; }
-          }
-          if (c == kNoChunk) {
-            c = oth_lo + (int)atomicAdd(oth_cnt, (unsigned)run);
-            if (c >= oth_hi) { c = kNoChunk; split_phase = 3; }
-          }
-        }
-        split_phase = __shfl_sync(0xffffffffu, split_phase, 0);
-        return __shfl_sync(0xffffffffu, c, 0);
-      }
-      if (split_phase == 3) return kNoChunk;
-    }
     if (lane == 0) c = (int)atomicAdd(P.work_counter, (unsigned)run);
     return __shfl_sync(0xffffffffu, c, 0);
   };
@@ -746,10 +704,6 @@ cudaError_t launch_persist(const WalkParams &p, long long n, cudaStream_t stream
   const unsigned grid = (unsigned)std::min<long long>(want, (long long)sms * occ);
   cudaError_t e = cudaMemsetAsync(p.work_counter, 0, sizeof(unsigned int), stream);
   if (e != cudaSuccess) return e;
-  if (GATHER != 0 && p.die0_sms > 0 && p.work_counter2) {
-    e = cudaMemsetAsync(p.work_counter2, 0, sizeof(unsigned int), stream);
-    if (e != cudaSuccess) return e;
-  }
   walk_persist_kernel<BLOCK, FETCH, MINB, REFILL_T, GATHER><<<grid, BLOCK, 0, stream>>>(p);
   return cudaGetLastError();
 }

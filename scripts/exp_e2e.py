@@ -1,6 +1,6 @@
 """End-to-end MoveToNextLocation from host memory (config c2): staged path (default) for several
 worker counts and chunk sizes, pageable vs pinned caller buffers, vs the direct path.
-Usage: python scripts/exp_e2e.py [mode ...]   mode = staged:<threads>:<chunk> | pinned:<threads>:<chunk> | registered:<t>:<c> | pinned_staged:<t>:<c> |
+Usage: python scripts/exp_e2e.py [mode ...]   mode = staged:<threads>:<chunk> | pinned_staged:<threads>:<chunk> |
                                                      direct_registered | direct_pageable | direct_pinned"""
 import sys, os, json, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -19,24 +19,21 @@ wl = SyntheticWorkload(box=box, num_particles=n, mean_length=cfg["mean_length"],
 init = wl.initial_positions().cpu().numpy()
 NB = int(os.environ.get("EXP_STEPS", 8))
 batches = [tuple(x.cpu().numpy() for x in wl.next_step()) for _ in range(NB)]
-modes = sys.argv[1:] or ["staged:0:0", "pinned:0:0", "direct_registered", "direct_pinned"]
+modes = sys.argv[1:] or ["staged:0:0", "pinned_staged:0:0", "direct_registered", "direct_pinned"]
 for mode in modes:
     parts = mode.split(":")
     kind = parts[0]
     eng = PumiTally.from_spec(f"box:{cells[0]},{cells[1]},{cells[2]}", n, device=0)
-    if kind in ("staged", "pinned", "registered", "pinned_staged"):
+    if kind in ("staged", "pinned_staged"):
         if len(parts) > 1 and int(parts[1]) > 0: eng.set_option("host_threads", int(parts[1]))
         if len(parts) > 2 and int(parts[2]) > 0: eng.set_option("chunk", int(parts[2]))
-        if kind == "registered": eng.set_option("register_host", 1)   # pageable arrays, page-locked by the engine
-        if kind in ("registered", "pinned"): eng.set_option("pinned_path", 1)  # DMA from the caller's arrays, positions mirrored back
-        if kind == "pinned_staged": eng.set_option("pinned_path", 0)  # pinned arrays through the staging slots (the default)
     else:
         eng.set_option("host_path", 0)
         eng.set_option("register_host", 1 if kind == "direct_registered" else 0)
     t0 = time.perf_counter()
     eng.CopyInitialPosition(init.reshape(-1))
     t_init = time.perf_counter() - t0
-    if kind in ("pinned", "pinned_staged", "direct_pinned"):
+    if kind in ("pinned_staged", "direct_pinned"):
         bufs = [torch.empty(s, dtype=d, pin_memory=True) for s, d in ((3 * n, torch.float64), (3 * n, torch.float64), (n, torch.int8), (n, torch.float64))]
         O, D, F, W = (b.numpy() for b in bufs)
     else:

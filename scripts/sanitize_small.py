@@ -16,9 +16,9 @@ for v in variants:
     e.set_option("chunk", 2048)  # several upload/compute ranges, ragged last chunk
     run_workload(e, OraclePumiTally(coords, t2v, wl.n), wl, steps=2, label=f"sanitize v{v}")
     print("variant", v, "staged host path ok", e.stats()["segments"], flush=True)
-    # direct host path, device-side state accessors, weight sum, normalisation, pinned-caller path
+    # direct host path, device-side state accessors, weight sum, normalisation, page-locked caller arrays
     import torch
-    for opts, pinned in (({"host_path": 0}, False), ({"host_path": 1, "pinned_path": 1}, True)):
+    for opts, pinned in (({"host_path": 0}, False), ({}, True)):
         coords, t2v, wl = box_case((6, 6, 5), 5003)
         e, orc = PumiTally.from_arrays(coords, t2v, wl.n), OraclePumiTally(coords, t2v, wl.n)
         e.set_option("variant", v)

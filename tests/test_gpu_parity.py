@@ -344,35 +344,6 @@ def test_staged_path_reused_buffers_ragged_sizes_and_flag_values(threads):
     assert st["h2d_bytes"] < 24 * n + 4 * 57 * n
 
 
-def test_staged_path_every_origin_changed_and_none_changed():
-    """Patch-list overflow (every origin differs from the previous destination -> the slice travels
-    whole) and the opposite extreme (no origin changed -> no origin bytes at all)."""
-    coords, t2v = kuhn_box(6, 6, 5)
-    n = 30_000
-    rng = np.random.default_rng(3)
-    e = gpu_engine(8, chunk=4096)(coords, t2v, n)
-    orc = OraclePumiTally(coords, t2v, n)
-    pos = rng.uniform(0.05, 4.95, size=(n, 3))
-    for x in (e, orc):
-        x.CopyInitialPosition(pos.reshape(-1).copy())
-    sent = [e.stats()["h2d_bytes"]]
-    prev = pos
-    for step in range(4):
-        origin = prev.copy() if step % 2 == 0 else rng.uniform(0.05, 4.95, size=(n, 3))
-        dest = np.clip(origin + rng.normal(0, 0.8, size=(n, 3)), [0.011, 0.013, 0.017], [4.987, 4.983, 4.979])
-        fly, w = np.ones(n, dtype=np.int8), rng.uniform(0.5, 1.0, n)
-        for x in (e, orc):
-            x.MoveToNextLocation(origin.reshape(-1).copy(), dest.reshape(-1).copy(), fly.copy(), w.copy())
-        prev = dest
-        sent.append(e.stats()["h2d_bytes"])
-    per_move = np.diff(sent) / n
-    assert abs(per_move[0] - 33) < 0.01 and abs(per_move[2] - 33) < 0.01   # nothing changed: no origin bytes
-    assert abs(per_move[1] - 57) < 0.01 and abs(per_move[3] - 57) < 0.01   # everything changed: slices sent whole
-    assert_flux_close(e.flux, orc.flux, "overflow / no-change extremes")
-    np.testing.assert_array_equal(e.elem_ids, orc.elem_ids)
-    np.testing.assert_array_equal(e.positions, orc.positions)
-
-
 def _host_buffers(n, kind):
     """The caller's four arrays: 'pinned' = page-locked by the caller (torch), else ordinary numpy."""
     if kind == "pinned":
@@ -383,20 +354,60 @@ def _host_buffers(n, kind):
     return [np.empty(3 * n), np.empty(3 * n), np.empty(n, dtype=np.int8), np.empty(n)]
 
 
+def _every_origin_changed_and_none_changed(buffers):
+    """Patch-list overflow (every origin differs from the previous destination -> the slice travels
+    whole) and the opposite extreme (no origin changed -> no origin bytes at all), staged from the
+    caller's `buffers` (_host_buffers kind)."""
+    coords, t2v = kuhn_box(6, 6, 5)
+    n = 30_000
+    rng = np.random.default_rng(3)
+    e = gpu_engine(8, chunk=4096)(coords, t2v, n)
+    e.set_option("host_path", 1)  # staged also for page-locked arrays, not the automatic choice
+    orc = OraclePumiTally(coords, t2v, n)
+    pos = rng.uniform(0.05, 4.95, size=(n, 3))
+    for x in (e, orc):
+        x.CopyInitialPosition(pos.reshape(-1).copy())
+    O, D, F, W = _host_buffers(n, buffers)
+    sent = [e.stats()["h2d_bytes"]]
+    prev = pos
+    for step in range(4):
+        origin = prev.copy() if step % 2 == 0 else rng.uniform(0.05, 4.95, size=(n, 3))
+        dest = np.clip(origin + rng.normal(0, 0.8, size=(n, 3)), [0.011, 0.013, 0.017], [4.987, 4.983, 4.979])
+        w = rng.uniform(0.5, 1.0, n)
+        O[:], D[:], W[:], F[:] = origin.reshape(-1), dest.reshape(-1), w, 1
+        e.MoveToNextLocation(O, D, F, W)
+        orc.MoveToNextLocation(origin.reshape(-1).copy(), dest.reshape(-1).copy(), np.ones(n, dtype=np.int8), w.copy())
+        prev = dest
+        sent.append(e.stats()["h2d_bytes"])
+    per_move = np.diff(sent) / n
+    assert abs(per_move[0] - 33) < 0.01 and abs(per_move[2] - 33) < 0.01   # nothing changed: no origin bytes
+    assert abs(per_move[1] - 57) < 0.01 and abs(per_move[3] - 57) < 0.01   # everything changed: slices sent whole
+    assert_flux_close(e.flux, orc.flux, f"overflow / no-change extremes, {buffers} buffers")
+    np.testing.assert_array_equal(e.elem_ids, orc.elem_ids)
+    np.testing.assert_array_equal(e.positions, orc.positions)
+
+
+def test_staged_path_every_origin_changed_and_none_changed():
+    _every_origin_changed_and_none_changed("pageable")
+
+
+def test_page_locked_caller_arrays_every_origin_changed_and_none_changed():
+    """Page-locked caller arrays go through the staging slots as well (host_path=1): the same 33 B /
+    57 B per particle as from pageable arrays."""
+    _every_origin_changed_and_none_changed("pinned")
+
+
 @pytest.mark.parametrize("kind", ["pinned", "registered"])
 @pytest.mark.parametrize("variant", [-1, 16, 24])
-def test_pinned_caller_path_matches_oracle(kind, variant):
-    """Host-pointer moves on page-locked caller arrays (pinned by the caller, or by register_host=1):
-    dest and weights are DMA'd from the caller's memory, origins are compared with the positions the
-    device sends back after every move, re-sourced particles are relocated by their own kernel.
-    Re-sourcing, hull clipping, non-flying particles, odd flag values, a device-pointer move in
-    between and non-finite origins included."""
+def test_page_locked_caller_arrays_match_oracle(kind, variant):
+    """Host-pointer moves through the default staged path on page-locked caller arrays (pinned by the
+    caller, or by register_host=1).  Re-sourcing, hull clipping, non-flying particles, odd flag values,
+    a device-pointer move in between and non-finite origins included."""
     import torch
 
     coords, t2v, wl = box_case((6, 6, 5), 60_007)
     n = wl.n
     e = gpu_engine(variant, chunk=8192)(coords, t2v, n)
-    e.set_option("pinned_path", 1)
     e.set_option("host_path", 1)  # not the automatic choice between staged and direct uploads
     if kind == "registered":
         e.set_option("register_host", 1)
@@ -413,11 +424,10 @@ def test_pinned_caller_path_matches_oracle(kind, variant):
         odd = rng.random(n) < 0.01
         f[odd] = rng.choice(np.array([2, -1, 127], dtype=np.int8), int(odd.sum()))
         f_ref = f.copy()
-        if step == 3:  # a device-pointer move: nothing comes back, the position mirror must be refreshed
+        if step == 3:  # a device-pointer move: the staging slots do not see it
             t = [torch.from_numpy(np.ascontiguousarray(x)).cuda() for x in (o, d, f, w)]
             e.move_device(*(x.data_ptr() for x in t), torch.cuda.current_stream().cuda_stream)
             torch.cuda.synchronize()
-            assert e.get_option("position_mirror") == 0
         else:
             if step == 4:  # unusable origins: those particles sit the move out and are counted
                 bad = np.flatnonzero(f == 1)[:25]
@@ -428,9 +438,8 @@ def test_pinned_caller_path_matches_oracle(kind, variant):
             O[:], D[:], W[:], F[:] = o.reshape(-1), d.reshape(-1), w, f
             e.MoveToNextLocation(O, D, F, W)
             assert not F.any()
-            assert e.get_option("position_mirror") == 1
         orc.MoveToNextLocation(np.nan_to_num(o, nan=0.5, posinf=0.5).reshape(-1).copy(), d.reshape(-1).copy(), f_ref, w.copy())
-        assert_flux_close(e.flux, orc.flux, f"pinned caller path, step {step}")
+        assert_flux_close(e.flux, orc.flux, f"page-locked caller arrays, step {step}")
         ok = np.ones(n, dtype=bool)
         if step == 4:
             ok[bad] = False  # the oracle was told they do not fly; here they were skipped: same state either way
@@ -438,38 +447,6 @@ def test_pinned_caller_path_matches_oracle(kind, variant):
         np.testing.assert_allclose(e.positions, orc.positions, rtol=0, atol=1e-9)
     st = e.stats()
     assert st["segments"] == orc.n_segments and st["lost"] == lost
-    assert e.get_option("d2h_bytes") == 5 * 24 * n
-
-
-def test_pinned_caller_path_every_origin_changed_and_none_changed():
-    coords, t2v = kuhn_box(6, 6, 5)
-    n = 30_000
-    rng = np.random.default_rng(3)
-    e = gpu_engine(8, chunk=4096)(coords, t2v, n)
-    e.set_option("pinned_path", 1)
-    e.set_option("host_path", 1)
-    orc = OraclePumiTally(coords, t2v, n)
-    pos = rng.uniform(0.05, 4.95, size=(n, 3))
-    for x in (e, orc):
-        x.CopyInitialPosition(pos.reshape(-1).copy())
-    O, D, F, W = _host_buffers(n, "pinned")
-    sent = [e.stats()["h2d_bytes"]]
-    prev = pos
-    for step in range(4):
-        origin = prev.copy() if step % 2 == 0 else rng.uniform(0.05, 4.95, size=(n, 3))
-        dest = np.clip(origin + rng.normal(0, 0.8, size=(n, 3)), [0.011, 0.013, 0.017], [4.987, 4.983, 4.979])
-        w = rng.uniform(0.5, 1.0, n)
-        O[:], D[:], W[:], F[:] = origin.reshape(-1), dest.reshape(-1), w, 1
-        e.MoveToNextLocation(O, D, F, W)
-        orc.MoveToNextLocation(origin.reshape(-1).copy(), dest.reshape(-1).copy(), np.ones(n, dtype=np.int8), w.copy())
-        prev = dest
-        sent.append(e.stats()["h2d_bytes"])
-    per_move = np.diff(sent) / n
-    assert abs(per_move[0] - 33) < 0.01 and abs(per_move[2] - 33) < 0.01   # nothing changed: no origin bytes
-    assert abs(per_move[1] - 57) < 0.01 and abs(per_move[3] - 57) < 0.01   # everything changed: slices sent whole
-    assert_flux_close(e.flux, orc.flux, "pinned path: overflow / no-change extremes")
-    np.testing.assert_array_equal(e.elem_ids, orc.elem_ids)
-    np.testing.assert_array_equal(e.positions, orc.positions)
 
 
 def test_page_locked_caller_arrays_get_the_faster_of_staged_and_direct_uploads():
@@ -1139,21 +1116,6 @@ def test_walks_cut_short_by_the_crossing_limit_are_reported_and_recoverable(vari
     assert_flux_close(eng.flux, orc2.flux, "after recovery")
     moved = f == 1  # particles that did not fly still sit on their face
     np.testing.assert_array_equal(eng.elem_ids[moved], orc2.elem_ids[moved])
-
-
-@pytest.mark.parametrize("variant", [16, 24])
-def test_die_split_of_the_sorted_kernels_keeps_results(variant):
-    """Option die_split=1: the SMs of each L2 partition take the sorted particles from their own end of the
-    sequence (two ticket counters + work stealing); every particle is still walked exactly once."""
-    coords, t2v, wl = box_case((8, 8, 8), 60_000)
-    e = gpu_engine(variant, chunk=16384)(coords, t2v, wl.n)
-    e.set_option("die_split", 1)
-    assert e.get_option("die_split") == 1
-    n0 = e.get_option("l2_partition0_sms")
-    assert n0 == 0 or 40 <= n0 <= 108  # a B200: 76 of 148; 0 = no two groups found (the split then stays off)
-    run_workload(e, OraclePumiTally(coords, t2v, wl.n), wl, steps=3, label=f"die split v{variant}")
-    st = e.stats()
-    assert st["lost"] == 0 and st["tracks"] > 0
 
 
 def test_autotuner_switches_kernels_without_changing_results():
