@@ -13,10 +13,13 @@
 // use the additive <pumitally/PumiTallyExtras.h>.
 //
 //   g++ -std=c++17 -I include examples/openmc_like_driver.cpp -L pumiumtally_b200/lib -lpumitally \
-//       -Wl,-rpath,$PWD/pumiumtally_b200/lib -o driver && ./driver box:20,20,20 1000000 20 [inactive_batches [energy_groups]]
+//       -Wl,-rpath,$PWD/pumiumtally_b200/lib -o driver && ./driver box:20,20,20 1000000 20 [inactive_batches [energy_groups [active_batches]]]
 //
 // energy_groups > 1 turns the tally into a filtered one (pumitally::SetScoreBins): each flight scores into the
 // flux array of the group it was sampled in; the VTK output then carries flux_bin<k> next to flux (their sum).
+// active_batches > 1 runs that many active batches of `sweeps` sweeps and closes each with pumitally::EndBatch:
+// the VTK output then holds the mean over the batches with its standard deviation (flux_std_dev), and the
+// driver prints the largest relative error of the tally (pumitally::MaxRelativeError, OpenMC's tally trigger).
 #include <chrono>
 #include <cmath>
 #include <cstdint>
@@ -46,6 +49,7 @@ int main(int argc, char **argv) {
   const int sweeps = argc > 3 ? std::atoi(argv[3]) : 10;
   const int inactive = argc > 4 ? std::atoi(argv[4]) : 0;  // batches of `sweeps` sweeps run and discarded first
   const int groups = argc > 5 ? std::atoi(argv[5]) : 1;    // energy groups of the score filter
+  const int active = argc > 6 ? std::atoi(argv[6]) : 1;    // active batches, each closed by EndBatch when > 1
   double box[3] = {20, 20, 20};
   if (mesh.rfind("box:", 0) == 0) std::sscanf(mesh.c_str() + 4, "%lf,%lf,%lf", &box[0], &box[1], &box[2]);
 
@@ -66,8 +70,9 @@ int main(int argc, char **argv) {
   if (inactive > 0) pumitally::SetSourceNormalization(tally, 3);
   const auto t0 = std::chrono::steady_clock::now();
   long long flights = 0, leaks = 0;
-  for (int batch = 0; batch <= inactive; ++batch) {
-  if (batch > 0) {  // an inactive batch ends: discard its tally, keep the particles where they are
+  const int batches = inactive + (active > 1 ? active : 1);
+  for (int batch = 0; batch < batches; ++batch) {
+  if (batch > 0 && batch <= inactive) {  // an inactive batch ends: discard its tally, keep the particles where they are
     pumitally::ResetTally(tally);
     flights = leaks = 0;
   }
@@ -94,11 +99,19 @@ int main(int argc, char **argv) {
     else
       tally.MoveToNextLocation(origin.data(), dest.data(), flying.data(), weight.data(), 3 * n);
   }
+  if (active > 1 && batch >= inactive && pumitally::EndBatch(tally)) return 1;  // an active batch ends
   }
   const double secs = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
   tally.WriteTallyResults();  // openmc_simulation_finalize
   std::printf("DRIVER_OK %lld flights (%lld leaked and re-sampled) in %d sweeps, %.3f s host loop + tally calls, "
               "source normalisation %.6f\n",
               flights, leaks, sweeps, secs, pumitally_get_source_normalization(pumitally::engine_of(tally)));
+  if (active > 1) {
+    double max_rel = 0.0;
+    int64_t where = -1, above = 0;
+    if (pumitally::MaxRelativeError(tally, 0.05, &max_rel, &where, &above)) return 1;
+    std::printf("TALLY_TRIGGER %d active batches: max relative error %.17g at %lld, %lld bins above 0.05\n", active,
+                max_rel, (long long)where, (long long)above);
+  }
   return 0;
 }

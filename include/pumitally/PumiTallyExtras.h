@@ -18,7 +18,7 @@ namespace pumitally {
 // nullptr if `tally` is not a live PumiTally object
 pumitally_engine *engine_of(const PumiTally &tally);
 
-// Start a new batch: zero the flux, the statistics and the initial-track weight.
+// Start over: zero the flux, the statistics, the batch statistics and the initial-track weight.
 inline int ResetTally(const PumiTally &tally) { return pumitally_reset_tally(engine_of(tally)); }
 
 // mode 0 volume only (reference behaviour), 1 / num_particles, 2 / value, 3 / total weight of the
@@ -34,6 +34,18 @@ inline int MoveToNextLocationBinned(const PumiTally &tally, double *particle_ori
                                     int8_t *flying, double *weights, const int32_t *bins, int32_t size) {
   return pumitally_move_to_next_location_binned(engine_of(tally), particle_origin, particle_destinations, flying,
                                                 weights, bins, size);
+}
+
+// Batch statistics (see pumitally_end_batch in pumitally_c.h): close the batch, read mean and standard
+// deviation of the mean per element (n = num_elements or nbins * num_elements), query the relative-error
+// trigger.  Collective on several GPUs.
+inline int EndBatch(const PumiTally &tally) { return pumitally_end_batch(engine_of(tally)); }
+inline int GetTallyStatistics(const PumiTally &tally, double *mean, double *std_dev, int64_t n) {
+  return pumitally_get_tally_statistics(engine_of(tally), mean, std_dev, n);
+}
+inline int MaxRelativeError(const PumiTally &tally, double threshold, double *max_rel, int64_t *index,
+                            int64_t *count_above) {
+  return pumitally_get_max_relative_error(engine_of(tally), threshold, max_rel, index, count_above);
 }
 
 }  // namespace pumitally

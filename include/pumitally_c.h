@@ -122,7 +122,7 @@ int pumitally_set_output_name(pumitally_engine *e, const char *filename);
  * (crossing limit per walk; 0 = number of elements + 16, the default), "l2_fetch", "autotune"
  * (1 = default: while "variant" is automatic the engine times the streaming and the sorted/packed
  * kernel on moves 1-4 of every 64 and keeps the faster one).  Read-only: "launches", "staged",
- * "stage_host_us", "stage_sent_bytes". */
+ * "stage_host_us", "stage_sent_bytes", "batches" (see pumitally_end_batch). */
 int pumitally_set_option(pumitally_engine *e, const char *name, int64_t value);
 int64_t pumitally_get_option(const pumitally_engine *e, const char *name);
 
@@ -200,6 +200,34 @@ int pumitally_move_to_next_location_device_binned(pumitally_engine *e, const dou
                                                   const double *d_destinations, const int8_t *d_flying,
                                                   const double *d_weights, const int32_t *d_bins,
                                                   int32_t size, void *stream);
+
+/* ---- additive: batch statistics ------------------------------------------
+ * Every Monte Carlo tally result is a mean over batches with the standard deviation of that mean; OpenMC
+ * keeps a running sum and sum of squares per bin over the active batches, and its tally triggers stop a
+ * run once the relative error falls below a threshold.  pumitally_end_batch closes the current batch:
+ * the raw flux since the last end_batch / pumitally_reset_tally / pumitally_set_score_bins /
+ * CopyInitialPosition (summed over ranks when a communicator exists, by the exchange pumitally_comm_init
+ * chose; an earlier pumitally_exchange_tally result is superseded) is divided by the batch's source
+ * divisor -- mode 0: 1; mode 1: the number of particles summed over ranks; mode 2: `value`, the global
+ * source weight of one batch; mode 3: the weight of the batch's first tracks summed over ranks -- and the
+ * result x is added to S1 and x*x to S2 per (bin, element); then the flux and the first-track weight start
+ * over.  A divisor that is not finite and > 0 makes the call fail and change nothing.  pumitally_stats keep
+ * counting; pumitally_reset_tally and pumitally_set_score_bins discard S1, S2 and the batch count n
+ * (pumitally_get_option "batches").  On several GPUs each rank keeps the sums of its share of the elements
+ * (the reduce-scatter layout of pumitally_reduce_tally_to_owners) and all three calls are COLLECTIVE.
+ * Moves may be on any stream: end_batch synchronises the device first and returns after its own pass. */
+int pumitally_end_batch(pumitally_engine *e);
+/* mean = S1 / n / volume and its standard deviation sqrt((S2/n - (S1/n)^2) / (n - 1)) / volume (a negative
+ * rounding residue is clamped to 0; NaN with n == 1), caller's element numbering; n as for
+ * pumitally_get_flux; either pointer may be NULL.  Fails before the first end_batch.  WriteTallyResults
+ * writes the mean as "flux" (with bins: "flux_bin<k>" and "flux" = their sum) and, from two batches on,
+ * "flux_std_dev" / "flux_bin<k>_std_dev"; moves after the last end_batch are not part of it. */
+int pumitally_get_tally_statistics(pumitally_engine *e, double *out_mean, double *out_std_dev, int64_t n);
+/* Tally trigger: over the (bin, element) pairs with a non-zero mean, the largest std_dev / |mean|, the index
+ * bin * num_elements + caller's element id where it is reached (lowest on ties), and how many pairs exceed
+ * `threshold` (no pair with a non-zero mean: 0, -1, 0).  Needs n >= 2; every rank gets the same answer. */
+int pumitally_get_max_relative_error(pumitally_engine *e, double threshold, double *out_max_rel,
+                                     int64_t *out_index, int64_t *out_count_above);
 
 /* test hook: processing order produced by the last binning pass (ids of flying particles
  * grouped by seed-grid cell); returns the number of entries, copies at most n of them */

@@ -22,6 +22,7 @@ LIB_EXP = os.path.join(LIBDIR, "libpumitally_exp.so")  # product + measured alte
 SOURCES = [
     "walk_kernels.cu",
     "bin_kernels.cu",
+    "batch_stats.cu",
     "engine.cu",
     "host_stage.cpp",
     "tet_mesh.cpp",

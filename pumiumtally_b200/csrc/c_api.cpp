@@ -252,6 +252,19 @@ int pumitally_reduce_tally_to_owners(pumitally_engine *e) {
   return guarded(e, [&](ptb::Engine &g) { return g.reduce_tally_to_owners(); });
 }
 
+int pumitally_end_batch(pumitally_engine *e) {
+  return guarded(e, [&](ptb::Engine &g) { return g.end_batch(); });
+}
+int pumitally_get_tally_statistics(pumitally_engine *e, double *out_mean, double *out_std_dev, int64_t n) {
+  return guarded(e, [&](ptb::Engine &g) { return g.get_tally_statistics(out_mean, out_std_dev, n); });
+}
+int pumitally_get_max_relative_error(pumitally_engine *e, double threshold, double *out_max_rel, int64_t *out_index,
+                                     int64_t *out_count_above) {
+  return guarded(e, [&](ptb::Engine &g) {
+    return g.max_relative_error(threshold, out_max_rel, out_index, out_count_above);
+  });
+}
+
 int64_t pumitally_debug_order(pumitally_engine *e, int32_t *out, int64_t n) {
   if (!e || !e->impl) return -1;
   return e->impl->debug_order(out, n);

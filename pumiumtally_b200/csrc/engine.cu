@@ -7,11 +7,13 @@
 #include <atomic>
 #include <chrono>
 #include <climits>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <stdexcept>
 
+#include "batch_stats.cuh"
 #include "host_stage.hpp"
 #include "seed_grid.hpp"
 #include "vtk_writer.hpp"
@@ -135,6 +137,7 @@ Engine::~Engine() {
   cudaDeviceSynchronize();
   if (nccl_comm_) nccl_comm_destroy(nccl_comm_);
   cudaFree(d_flux_global_);
+  release_batch_buffers();
   if (ev_order_) cudaEventDestroy(ev_order_);
   if (ev_done_) cudaEventDestroy(ev_done_);
   if (ev_bins_) cudaEventDestroy(ev_bins_);
@@ -852,6 +855,7 @@ int Engine::set_score_bins(int32_t nbins) {
   d_flux_ = nf;
   flux_alloc_ = len;
   nbins_ = nbins;
+  release_batch_buffers();  // sized for the old number of bins
   if (nbins > 1 && !d_mask_) {
     PTB_CUDA_OK(cudaMalloc(reinterpret_cast<void **>(&d_mask_), std::max<size_t>(size_t(n_), 16)));
     PTB_CUDA_OK(cudaMalloc(reinterpret_cast<void **>(&d_bins_), std::max<size_t>(size_t(n_), 4) * sizeof(int32_t)));
@@ -1060,6 +1064,7 @@ int Engine::reset_tally() {
   kernel_ms_ = 0.0;
   h2d_bytes_ = 0.0;
   moves_ = 0;
+  batches_ = 0;  // the next end_batch starts the sums over (no need to clear them)
   return 0;
 }
 
@@ -1110,6 +1115,7 @@ int64_t Engine::get_option(const std::string &name) const {
   }
   if (name == "allreduce_us") return int64_t(allreduce_ms_ * 1e3);  // device time of the last batch-end exchange
   if (name == "score_bins") return nbins_;
+  if (name == "batches") return int64_t(batches_);  // batches closed by end_batch since the last reset
   if (name == "exchange_choice") return exchange_choice_;  // what exchange_tally() does: 0 all-reduce, 1 reduce-scatter
   if (name == "exchange_allreduce_us") return int64_t(exchange_ms_[0] * 1e3);  // comm_init's measurement of the two
   if (name == "exchange_reduce_scatter_us") return int64_t(exchange_ms_[1] * 1e3);
@@ -1203,24 +1209,188 @@ int64_t Engine::debug_order(int32_t *out, int64_t n) {
 // FinalizeTallies (PumiTallyImpl.cpp:411-416)
 int Engine::write_tally_results() {
   const size_t E = size_t(mesh_.ntets);
-  std::vector<double> nf(E * size_t(nbins_)), vol(E);
-  if (get_normalized_flux(nf.data(), vol.data(), int64_t(nf.size()))) return 1;  // caller's element order
+  std::vector<double> nf(E * size_t(nbins_)), vol(E), sd;
+  if (batches_ > 0) {
+    // after end_batch: the mean over the ended batches (moves since the last one are not part of the result)
+    // and, from two batches on, its standard deviation
+    if (batches_ >= 2) sd.resize(nf.size());
+    if (get_tally_statistics(nf.data(), sd.empty() ? nullptr : sd.data(), int64_t(nf.size()))) return 1;
+    for (size_t i = 0; i < E; ++i) vol[mesh_.orig_of_internal[i]] = mesh_.volume[i];
+  } else if (get_normalized_flux(nf.data(), vol.data(), int64_t(nf.size()))) {  // caller's element order
+    return 1;
+  }
   // filtered tally: "flux" is the sum over the bins (what the unfiltered tally would hold), and every
-  // bin is written as "flux_bin<k>" next to it
+  // bin is written as "flux_bin<k>" next to it (the sum gets no standard deviation: that would need the
+  // covariances between the bins)
   std::vector<std::pair<std::string, const double *>> extra;
   std::vector<double> per_bin;
   if (nbins_ > 1) {
     per_bin.assign(nf.begin(), nf.end());
-    for (int32_t b = 0; b < nbins_; ++b) extra.emplace_back("flux_bin" + std::to_string(b), per_bin.data() + size_t(b) * E);
+    for (int32_t b = 0; b < nbins_; ++b) {
+      extra.emplace_back("flux_bin" + std::to_string(b), per_bin.data() + size_t(b) * E);
+      if (!sd.empty()) extra.emplace_back("flux_bin" + std::to_string(b) + "_std_dev", sd.data() + size_t(b) * E);
+    }
     for (int32_t b = 1; b < nbins_; ++b)
       for (size_t i = 0; i < E; ++i) nf[i] += nf[size_t(b) * E + i];
     nf.resize(E);
+  } else if (!sd.empty()) {
+    extra.emplace_back("flux_std_dev", sd.data());
   }
   std::string err;
   if (!write_vtk_dataset(output_name_, mesh_, nf, vol, rank_, nranks_, &err, extra)) {
     fprintf(stderr, "[pumitally] ERROR: %s\n", err.c_str());
     return 1;
   }
+  return 0;
+}
+
+// ------------------------------------------------------------------ batch statistics
+
+size_t Engine::stats_count() const {
+  const size_t off = stats_offset(), len = flux_len();
+  return off >= len ? 0 : std::min(stats_len(), len - off);
+}
+
+// Allocated at the first end_batch, so that engines that never end a batch keep their memory footprint.
+int Engine::ensure_batch_buffers() {
+  if (d_s1_) return 0;
+  const size_t len = std::max<size_t>(stats_len(), 1);
+  const size_t small = 3 * size_t(kBatchTriggerBlocks) + 3 + 3 * size_t(std::max(nranks_, 1)) + 2;
+  if (cudaMalloc(reinterpret_cast<void **>(&d_s1_), len * sizeof(double)) != cudaSuccess ||
+      cudaMalloc(reinterpret_cast<void **>(&d_s2_), len * sizeof(double)) != cudaSuccess ||
+      cudaMalloc(reinterpret_cast<void **>(&d_batch_small_), small * sizeof(double)) != cudaSuccess) {
+    cudaGetLastError();
+    fprintf(stderr, "[pumitally] ERROR: no device memory for the batch statistics (%zu MB)\n", (2 * len * sizeof(double)) >> 20);
+    release_batch_buffers();
+    return 1;
+  }
+  batches_ = 0;
+  return 0;
+}
+
+void Engine::release_batch_buffers() {
+  cudaFree(d_s1_);
+  cudaFree(d_s2_);
+  cudaFree(d_batch_small_);
+  d_s1_ = d_s2_ = d_batch_small_ = nullptr;
+  batches_ = 0;
+}
+
+// The batch's source divisor: 1 (mode 0), the number of particles (1), the caller's value (2: the global
+// source weight of one batch), the weight of the batch's first tracks (3).  Particles and weights are summed
+// over the ranks (collective), unlike get_normalized_flux's per-rank divisor.
+int Engine::batch_divisor(double *out) {
+  double v = 1.0;
+  if (norm_mode_ == 1) v = double(n_);
+  else if (norm_mode_ == 2) v = norm_value_;
+  else if (norm_mode_ == 3) PTB_CUDA_OK(cudaMemcpy(&v, d_initial_weight_, sizeof(double), cudaMemcpyDeviceToHost));
+  if (nccl_comm_ && (norm_mode_ == 1 || norm_mode_ == 3)) {
+    double *d = d_batch_small_ + 3 * size_t(kBatchTriggerBlocks) + 3 + 3 * size_t(nranks_);
+    PTB_CUDA_OK(cudaMemcpyAsync(d, &v, sizeof(double), cudaMemcpyHostToDevice, compute_));
+    if (nccl_allreduce_sum_f64(nccl_comm_, d, d + 1, 1, compute_)) return 1;
+    PTB_CUDA_OK(cudaMemcpyAsync(&v, d + 1, sizeof(double), cudaMemcpyDeviceToHost, compute_));
+    PTB_CUDA_OK(cudaStreamSynchronize(compute_));
+  }
+  *out = v;
+  return 0;
+}
+
+// Ordering: the device synchronisation at the start puts every kernel of earlier moves, on whichever stream
+// they were enqueued, before the accumulate pass, and the pass has finished when the call returns, so every
+// later move comes after it.
+int Engine::end_batch() {
+  PTB_CUDA_OK(cudaSetDevice(device_));
+  if (synchronize() || ensure_batch_buffers()) return 1;
+  double div = 0.0;
+  if (batch_divisor(&div)) return 1;
+  if (!(std::isfinite(div) && div > 0.0)) {
+    fprintf(stderr, "[pumitally] ERROR: end_batch: the batch's source divisor (normalisation mode %d) is %g%s; "
+                    "nothing was accumulated\n", norm_mode_, div,
+            norm_mode_ == 3 ? " (no flying particle with a weight in the batch's first move)" : "");
+    return 1;
+  }
+  const double *x = d_flux_;
+  double *zero = d_flux_;  // one GPU: the pass clears the tally it reads
+  if (nccl_comm_) {
+    if (exchange_tally()) return 1;
+    x = d_flux_global_ + stats_offset();  // this rank's share of the sum over ranks
+    zero = nullptr;
+    PTB_CUDA_OK(cudaMemsetAsync(d_flux_, 0, flux_alloc_ * sizeof(double), compute_));
+  } else if (flux_alloc_ > flux_len()) {  // the unreported bin and the pad
+    PTB_CUDA_OK(cudaMemsetAsync(d_flux_ + flux_len(), 0, (flux_alloc_ - flux_len()) * sizeof(double), compute_));
+  }
+  PTB_CUDA_OK(launch_batch_accumulate(x, div, zero, d_s1_, d_s2_, int64_t(stats_count()), batches_ == 0, compute_));
+  PTB_CUDA_OK(cudaMemsetAsync(d_initial_weight_, 0, sizeof(double), compute_));
+  PTB_CUDA_OK(cudaStreamSynchronize(compute_));
+  initial_weight_pending_ = true;
+  flux_global_valid_ = flux_owned_only_ = false;
+  ++batches_;
+  return 0;
+}
+
+int Engine::get_tally_statistics(double *out_mean, double *out_std_dev, int64_t n) {
+  const int64_t E = mesh_.ntets;
+  if (n != E && n != int64_t(nbins_) * E) return 1;
+  if (batches_ == 0) {
+    fprintf(stderr, "[pumitally] ERROR: tally statistics before the first end_batch\n");
+    return 1;
+  }
+  if (synchronize()) return 1;
+  // the finish pass writes this rank's share of both arrays, the all-gather (collective) the others
+  const size_t full = nccl_comm_ ? share_ * size_t(nranks_) : flux_len(), off = stats_offset();
+  double *d_out = nullptr;
+  PTB_CUDA_OK(cudaMalloc(reinterpret_cast<void **>(&d_out), 2 * std::max<size_t>(full, 1) * sizeof(double)));
+  std::unique_ptr<double, cudaError_t (*)(void *)> keep(d_out, cudaFree);
+  double *d_mean = d_out, *d_std = d_out + full;
+  PTB_CUDA_OK(launch_batch_finish(d_s1_, d_s2_, int64_t(stats_count()), int64_t(off), E, d_volume_, double(batches_),
+                                  d_mean + off, d_std + off, compute_));
+  if (nccl_comm_ && (nccl_all_gather_f64(nccl_comm_, d_mean + off, d_mean, share_, compute_) ||
+                     nccl_all_gather_f64(nccl_comm_, d_std + off, d_std, share_, compute_)))
+    return 1;
+  PTB_CUDA_OK(cudaStreamSynchronize(compute_));
+  std::vector<double> tmp(static_cast<size_t>(n));
+  const std::pair<double *, const double *> outs[2] = {{out_mean, d_mean}, {out_std_dev, d_std}};
+  for (const auto &o : outs) {
+    if (!o.first) continue;
+    PTB_CUDA_OK(cudaMemcpy(tmp.data(), o.second, size_t(n) * sizeof(double), cudaMemcpyDeviceToHost));
+    for (int64_t b = 0; b * E < n; ++b)
+      for (int64_t i = 0; i < E; ++i) o.first[b * E + mesh_.orig_of_internal[i]] = tmp[b * E + i];  // caller's numbering
+  }
+  return 0;
+}
+
+// Tally trigger: each rank reduces its share to one (max, index, count) record, the records are gathered
+// and combined the same way on every rank.
+int Engine::max_relative_error(double threshold, double *max_rel, int64_t *index, int64_t *count_above) {
+  if (batches_ < 2) {
+    fprintf(stderr, "[pumitally] ERROR: the relative error needs at least two ended batches (have %llu)\n",
+            (unsigned long long)batches_);
+    return 1;
+  }
+  if (synchronize() || ensure_element_maps()) return 1;
+  double *rec = d_batch_small_ + 3 * size_t(kBatchTriggerBlocks), *all = rec + 3;
+  PTB_CUDA_OK(launch_batch_trigger(d_s1_, d_s2_, int64_t(stats_count()), int64_t(stats_offset()), mesh_.ntets,
+                                   d_volume_, d_orig_of_internal_, double(batches_), threshold, d_batch_small_, rec,
+                                   compute_));
+  const int nrec = nccl_comm_ ? nranks_ : 1;
+  if (nccl_comm_ && nccl_all_gather_f64(nccl_comm_, rec, all, 3, compute_)) return 1;
+  std::vector<double> h(3 * size_t(nrec));
+  PTB_CUDA_OK(cudaMemcpyAsync(h.data(), nccl_comm_ ? all : rec, h.size() * sizeof(double), cudaMemcpyDeviceToHost, compute_));
+  PTB_CUDA_OK(cudaStreamSynchronize(compute_));
+  double best = -1.0, cnt = 0.0;
+  int64_t best_idx = -1;
+  for (int r = 0; r < nrec; ++r) {
+    const double rel = h[3 * size_t(r)];
+    const int64_t idx = int64_t(h[3 * size_t(r) + 1]);
+    cnt += h[3 * size_t(r) + 2];
+    if (rel >= 0.0 && (rel > best || (rel == best && idx < best_idx))) {
+      best = rel;
+      best_idx = idx;
+    }
+  }
+  if (max_rel) *max_rel = best < 0.0 ? 0.0 : best;
+  if (index) *index = best_idx;
+  if (count_above) *count_above = int64_t(cnt);
   return 0;
 }
 
@@ -1232,6 +1402,7 @@ int Engine::comm_init(int rank, int nranks, const uint8_t id[128]) {
   if (nccl_comm_init_rank(&nccl_comm_, nranks, id, rank)) return 1;
   rank_ = rank;
   nranks_ = nranks;
+  release_batch_buffers();  // from here on every rank keeps the statistics of its share only
   // NCCL sets up its NVLink connections lazily inside the first collective: pay that here,
   // on the scratch array, not in the first batch-end exchange
   if (nranks < 1 || size_t(nranks) > kFluxPad) return 1;

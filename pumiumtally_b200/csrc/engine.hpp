@@ -91,6 +91,18 @@ class Engine {
   // whichever of the two comm_init measured to be quicker on this mesh (same choice on every rank)
   int exchange_tally();
 
+  // Batch statistics (batch_stats.cu).  end_batch closes the batch: the tally since the last end_batch /
+  // reset (summed over ranks through exchange_tally when a communicator exists), divided by the batch's
+  // source divisor, is added to S1 and its square to S2 per (bin, element), and the tally and the first-track
+  // weight start over.  Each rank keeps the sums of its share of the reduce-scatter layout only.  All three
+  // calls are collective on several GPUs.
+  int end_batch();
+  // mean = S1 / n / volume and the standard deviation of the mean, caller's numbering; n as for get_flux
+  int get_tally_statistics(double *out_mean, double *out_std_dev, int64_t n);
+  // largest std_dev / |mean| over the pairs with a non-zero mean, its bin * E + caller's element id, and how
+  // many pairs exceed `threshold` (no such pair: 0, -1, 0)
+  int max_relative_error(double threshold, double *max_rel, int64_t *index, int64_t *count_above);
+
  private:
   int launch_range(const double *d_origin, const double *d_dest, const int8_t *d_flying,
                    const double *d_weights, int32_t begin, int32_t end, cudaStream_t stream,
@@ -240,6 +252,18 @@ class Engine {
   int gather_shares();
   double *flux_view() { return flux_global_valid_ ? d_flux_global_ : d_flux_; }
   double allreduce_ms_ = 0.0;  // device time of the last exchange
+
+  // batch statistics: running sums over the ended batches of this rank's share of the bin-major tally
+  // (entries [stats_offset(), stats_offset() + stats_count()) of it), allocated at the first end_batch
+  uint64_t batches_ = 0;
+  double *d_s1_ = nullptr, *d_s2_ = nullptr;
+  double *d_batch_small_ = nullptr;  // trigger partials and records, the divisor sum
+  size_t stats_len() const { return nccl_comm_ ? share_ : flux_len(); }
+  size_t stats_offset() const { return nccl_comm_ ? size_t(rank_) * share_ : 0; }
+  size_t stats_count() const;
+  int ensure_batch_buffers();
+  void release_batch_buffers();
+  int batch_divisor(double *out);
   cudaEvent_t ev_ar0_ = nullptr, ev_ar1_ = nullptr;
 };
 

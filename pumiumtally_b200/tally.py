@@ -74,6 +74,10 @@ C_API = {
     "pumitally_allreduce_tally": (C.c_int, [C.c_void_p]),
     "pumitally_reduce_tally_to_owners": (C.c_int, [C.c_void_p]),
     "pumitally_exchange_tally": (C.c_int, [C.c_void_p]),
+    "pumitally_end_batch": (C.c_int, [C.c_void_p]),
+    "pumitally_get_tally_statistics": (C.c_int, [C.c_void_p, _dp, _dp, C.c_int64]),
+    "pumitally_get_max_relative_error": (
+        C.c_int, [C.c_void_p, C.c_double, _dp, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "pumitally_debug_order": (C.c_int64, [C.c_void_p, _ip, C.c_int64]),
     "pumitally_debug_stage": (C.c_int64, [_dp, _dp, _bp, _dp, _dp, _dp, _bp, C.c_int64, C.c_int32, C.c_int32,
                                           C.c_void_p, C.c_int64]),
@@ -318,6 +322,28 @@ class PumiTally:
 
     def source_normalization(self) -> float:
         return float(self._L.pumitally_get_source_normalization(self._h))
+
+    # ---- batch statistics --------------------------------------------------------
+    def end_batch(self):
+        """Close the batch: its normalised tally joins the running sums, the tally starts over (collective)."""
+        if self._L.pumitally_end_batch(self._h):
+            raise RuntimeError("end_batch failed")
+
+    def tally_statistics(self):
+        """(mean, std_dev) over the ended batches, per unit volume: shape (E,), or (nbins, E) with score bins."""
+        nb = self.score_bins
+        shape = (self.num_elements,) if nb == 1 else (nb, self.num_elements)
+        mean, std = np.empty(shape), np.empty(shape)
+        if self._L.pumitally_get_tally_statistics(self._h, mean.ctypes.data_as(_dp), std.ctypes.data_as(_dp), mean.size):
+            raise RuntimeError("get_tally_statistics failed")
+        return mean, std
+
+    def max_relative_error(self, threshold: float):
+        """(max std_dev/|mean|, bin * E + element id where it is reached, pairs above threshold); n >= 2."""
+        r, i, c = C.c_double(), C.c_int64(), C.c_int64()
+        if self._L.pumitally_get_max_relative_error(self._h, float(threshold), C.byref(r), C.byref(i), C.byref(c)):
+            raise RuntimeError("get_max_relative_error failed")
+        return r.value, i.value, c.value
 
     def set_option(self, name: str, value: int):
         if self._L.pumitally_set_option(self._h, name.encode(), int(value)):
